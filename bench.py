@@ -224,6 +224,37 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_BYTES = 60_000_000     # --dump-outputs: array data in all (with the .npy headers, under 64 MB)
+
+
+def dump_outputs(eng, out_dir: str):
+    """--dump-outputs: what a caller of the timed path receives from `eng`'s last run, as out_dir/<name>.npy in float32 or
+    float64 (the integer columns of the structured tables widened to float64, which holds them exactly); a table without
+    rows is not written.  An array larger than its share of DUMP_BYTES is a fixed, seeded sample of its rows in row order
+    (of the C2 workload: the dB spectrum), so that two builds run with the same arguments can be compared file for file."""
+    eng.download()
+    eng.sync()
+    r = eng.result(None)
+
+    def table(a):
+        return np.stack([a[f].astype(np.float64) for f in a.dtype.names], axis=1)
+
+    arrays = {"counts": table(eng.counts_table()), "segments": table(r.segments), "syllables": table(r.syllables),
+              "formants": r.formants, "energy": r.energy, "features": r.features}
+    if eng.cfg.want_spectrum:
+        arrays["spectrum"] = eng.spectrum(None)
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BYTES // len(arrays)     # a share per output of the configuration: a sample never depends on other row counts
+    for name, a in arrays.items():
+        if len(a) == 0:                 # a table this output level does not fill (syllables at level 5, the C2 workload)
+            continue
+        a = np.ascontiguousarray(a, np.float64 if a.dtype == np.float64 else np.float32)
+        if a.nbytes > cap:
+            keep = np.random.default_rng(20261017).choice(len(a), cap // (a.nbytes // len(a)), replace=False)
+            a = a[np.sort(keep)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def cpu_port_run(cfg, pcms, threads: int):
     """The CPU oracle over the batch, OpenMP over utterances.  Returns (seconds, frames)."""
     from oracle import oracle
@@ -370,6 +401,8 @@ def run_c3(args, world, rank, local):
     barrier()
     ms_max = max_over_ranks(ev0.elapsed_time(ev1))
     launches_per_step = eng.launches
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, args.dump_outputs)
     stage_acc = np.zeros(5)
     eng.set_pipeline(1)
     eng.run_resident()
@@ -594,7 +627,12 @@ def main():
     ap.add_argument("--depth", type=int, default=4,
                     help="batches in flight: one handle + stream per batch slot, steps alternate between them so that batch "
                          "i+1's spectrum kernels overlap batch i's (latency-bound) segment scan and PCIe copies")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy, float32 / float64, "
+                         "at most 64 MB in all: a larger array is a fixed, seeded sample of its rows")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     capture_stdout()
     if args.impl == "reference":
         return run_reference(args)
@@ -664,6 +702,8 @@ def main():
     barrier()
     ms = ev0.elapsed_time(ev1)
     launches_per_step = eng.launches
+    if args.dump_outputs and rank == 0:
+        dump_outputs(engs[(args.steps - 1) % depth], args.dump_outputs)
     # per-stage CUDA-event times (recorded inside the library on the launching stream): a second timed region in
     # SERIAL mode (one sub-batch), because with the sub-batch pipeline the stages of different sub-batches overlap
     eng.set_pipeline(1)

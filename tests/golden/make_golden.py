@@ -27,6 +27,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 
+import npzparts  # noqa: E402
 from oracle import oracle  # noqa: E402
 from webspeechanalyzer_b200 import FaConfig  # noqa: E402
 from webspeechanalyzer_b200.engine import synth_speech  # noqa: E402
@@ -75,7 +76,7 @@ def main():
     np.savez_compressed(os.path.join(HERE, "sample_excerpt.npz"), **out)
     # the whole demo file (BASELINE config 1 input) as int16, so that the -m gpu tests can run C1 in full on the GPU
     # box, where /root/reference does not exist
-    np.savez_compressed(os.path.join(HERE, "sample_full_pcm.npz"), pcm_i16=i16, sample_rate=np.int32(sr))
+    npzparts.save(os.path.join(HERE, "sample_full_pcm"), {"pcm_i16": i16, "sample_rate": np.int32(sr)})
     json.dump(full, open(os.path.join(HERE, "sample_full.json"), "w"), indent=1)
 
     synth = {"cases": []}

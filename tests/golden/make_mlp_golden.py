@@ -13,6 +13,8 @@ import sys
 
 import numpy as np
 
+import npzparts
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
@@ -59,7 +61,7 @@ def main():
                                    "labels": m["labels"], "weights_sha256": shas[db],
                                    "same_weights_as": [k for k, v in shas.items() if v == shas[db]],
                                    "argmax_histogram": np.bincount(exp.argmax(axis=1), minlength=m["dims"][-1]).tolist()}
-    np.savez_compressed(os.path.join(HERE, "mlp_shipped.npz"), **out)
+    npzparts.save(os.path.join(HERE, "mlp_shipped"), out)
     json.dump(info, open(os.path.join(HERE, "mlp_shipped.json"), "w"), indent=1)
     print(json.dumps(info, indent=1))
 

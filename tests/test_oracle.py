@@ -10,6 +10,7 @@ from conftest import GOLDEN, sha
 from hypothesis import given, settings, strategies as st
 
 sys.path.insert(0, GOLDEN)
+import npzparts  # noqa: E402
 from framegen import adversarial_frames, voiced_random_frames  # noqa: E402
 
 from oracle import oracle  # noqa: E402
@@ -95,16 +96,13 @@ def test_row_width_and_identities():
 
 
 def test_feature_ranges_against_model_meta(sample_full):
-    meta = "/root/reference/dist/nnmodel/1/cats_emotion/model_meta.json"
-    if not os.path.exists(meta):
-        pytest.skip("reference not mounted")
-    rng = json.load(open(meta))["inputs"]
-    import wave
-    w = wave.open("/root/reference/samples/263771femaleprotagonist.wav")
-    pcm = np.frombuffer(w.readframes(w.getnframes()), np.int16).astype(np.float32) / 32768.0
-    _, an = oracle.analyze_pcm(FaConfig.default(output_level=13, window_step_ms=15.0), pcm, w.getframerate())
-    lo = np.array([rng[str(i)]["min"] for i in range(53)])
-    hi = np.array([rng[str(i)]["max"] for i in range(53)])
+    # the input ranges of the app's model 1 (dist/nnmodel/1/cats_emotion/model_meta.json, stored by make_mlp_golden.py)
+    # and the demo WAV's PCM (make_golden.py)
+    meta = npzparts.load(os.path.join(GOLDEN, "mlp_shipped"))
+    wav = npzparts.load(os.path.join(GOLDEN, "sample_full_pcm"))
+    pcm = wav["pcm_i16"].astype(np.float32) / 32768.0
+    _, an = oracle.analyze_pcm(FaConfig.default(output_level=13, window_step_ms=15.0), pcm, int(wav["sample_rate"]))
+    lo, hi = meta["m1_min"], meta["m1_max"]
     # the real-data ranges of 74 249 syllables bound ours on the demo file (small slack on the open-ended ones)
     inside = (an.features >= lo - 1e-9) & (an.features <= hi * 1.25 + 1e-9)
     assert inside.mean() > 0.99, np.argwhere(~inside)

@@ -176,7 +176,10 @@ def test_shipped_models_against_float64():
     (tests/golden/make_mlp_golden.py): same arg-max on every row, class scores within 1e-5.  Model 4 (53-512-512-8, 1.2 MB of
     parameters) takes the kernel variant that reads the parameters from L2 instead of shared memory."""
     here = os.path.dirname(os.path.abspath(__file__))
-    z = np.load(os.path.join(here, "golden", "mlp_shipped.npz"))
+    import sys
+    sys.path.insert(0, os.path.join(here, "golden"))
+    import npzparts
+    z = npzparts.load(os.path.join(here, "golden", "mlp_shipped"))
     info = json.load(open(os.path.join(here, "golden", "mlp_shipped.json")))
     rows = z["rows"]
     assert rows.shape == (info["rows"], 53) and rows.shape[0] >= 30

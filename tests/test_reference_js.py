@@ -14,6 +14,7 @@ import pytest
 from conftest import GOLDEN, sha
 
 sys.path.insert(0, GOLDEN)
+import npzparts  # noqa: E402
 from framegen import adversarial_frames, dropped_segment_frames, voiced_random_frames  # noqa: E402
 
 from oracle import oracle  # noqa: E402
@@ -35,7 +36,7 @@ _wav = {}
 def frames_for(inp, cfg):
     if inp["kind"] == "wav_full":
         if not _wav:
-            g = np.load(os.path.join(GOLDEN, "sample_full_pcm.npz"))
+            g = npzparts.load(os.path.join(GOLDEN, "sample_full_pcm"))
             _wav["pcm"], _wav["sr"] = g["pcm_i16"].astype(np.float32) / 32768.0, int(g["sample_rate"])
         return oracle.frontend(cfg, _wav["pcm"], _wav["sr"], spectrum=False)["frames"]
     if inp["kind"] == "synth":
