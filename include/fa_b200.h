@@ -311,6 +311,31 @@ FA_API const char* fa_mlp_last_error(const fa_mlp* m);
 FA_API int fa_mlp_classify(fa_mlp* m, const double* rows, size_t n_rows, float* probs);
 FA_API int fa_mlp_classify_features(fa_mlp* m, fa_handle* h, int64_t utt_id, float* probs, size_t cap_rows);
 
+/* ---- training of such a classifier on feature rows (K9, csrc/fa_train.cu; the algorithm is defined in DESIGN.md "K9") ----
+ * Trains n_jobs independent models of one architecture (hidden layers linear / relu / sigmoid, softmax output, categorical
+ * cross-entropy on integer labels) in one launch, without the host between steps.  The jobs share the row table `rows`
+ * (n_rows x dims[0] doubles), its `labels` (int32 in [0, dims[n_layers])) and the options; job j trains on the row indices
+ * row_idx[job_offsets[j] .. job_offsets[j + 1]) (repeats oversample, disjoint lists give folds), from its own seed and
+ * initial parameters.  Parameter layout (init_params, out_params): per job, K7's -- for each layer the kernel [in][out],
+ * then the bias, float32.  in_ranges NULL: each job's input ranges are the min / max of its own rows (a constant column
+ * gets max = min + 1); otherwise [n_jobs][2][dims[0]] (min row, then max row) used as given.  out_ranges has that shape,
+ * out_history is [n_jobs][epochs][2]: the row-weighted mean loss and the arg-max accuracy of every epoch.  Returns FA_OK,
+ * FA_ERR_INVALID_ARG with a message in err (labels, indices, empty jobs, options, non-softmax output, non-finite values in
+ * a selected row), FA_ERR_NO_DEVICE without an sm_100 device, or FA_ERR_CUDA / FA_ERR_OUT_OF_MEMORY. */
+#define FA_OPT_SGD 0
+#define FA_OPT_ADAM 1 /* beta1 0.9, beta2 0.999, epsilon 1e-7, bias-corrected (tf.js defaults) */
+typedef struct fa_train_opts {
+  double learning_rate;
+  int optimizer;        /* FA_OPT_SGD / FA_OPT_ADAM */
+  int epochs;           /* >= 0 */
+  int batch_size;       /* >= 1; the last batch of an epoch holds the remaining rows and averages over them */
+} fa_train_opts;
+FA_API int fa_mlp_train(int n_layers, const int* dims /* n_layers + 1 */, const int* activations, const double* rows,
+                        size_t n_rows, const int32_t* labels, int n_jobs, const int64_t* job_offsets /* n_jobs + 1 */,
+                        const int32_t* row_idx, const uint64_t* seeds, const float* init_params, const double* in_ranges,
+                        const fa_train_opts* opts, int device, float* out_params, double* out_ranges, double* out_history,
+                        char* err, size_t err_cap);
+
 FA_API int fa_copy_peak_candidates(fa_handle* h, int64_t utt_id, uint32_t* packed, int32_t* counts, size_t cap_rows,
                             int32_t* max_per_frame);
 

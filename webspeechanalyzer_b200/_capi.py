@@ -8,7 +8,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 
-from ._ctypes_defs import FaConfig, FaCounts, FaSegment, FaSyllable
+from ._ctypes_defs import FaConfig, FaCounts, FaSegment, FaSyllable, FaTrainOpts
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libfa_b200.so")
@@ -25,7 +25,7 @@ EXPORTS = [
     "fa_total_counts", "fa_copy_counts_table", "fa_pcie_probe", "fa_copy_spectrum", "fa_copy_spectrum_raw", "fa_copy_frames", "fa_copy_segments", "fa_copy_formants", "fa_copy_energy",
     "fa_copy_syllables", "fa_copy_features", "fa_copy_utterance_features", "fa_copy_curve_features", "fa_copy_track_points", "fa_set_truncate", "fa_mlp_create", "fa_mlp_destroy", "fa_mlp_last_error",
     "fa_mlp_classify", "fa_mlp_classify_features", "fa_copy_peak_candidates", "fa_copy_gsum", "fa_hop_samples", "fa_frames_for",
-    "fa_spec_bands", "fa_host_alloc", "fa_host_free",
+    "fa_spec_bands", "fa_host_alloc", "fa_host_free", "fa_mlp_train",
 ]
 SYNTH_EXPORTS = ["fa_synth_speech", "fa_synth_speech_i16_batch"]   # include/fa_synth.h -> libfa_synth.so (host-only generator)
 
@@ -88,6 +88,9 @@ def lib() -> C.CDLL:
     L.fa_mlp_last_error.argtypes = [H]; L.fa_mlp_last_error.restype = C.c_char_p
     L.fa_mlp_classify.argtypes = [H, C.c_void_p, C.c_size_t, C.c_void_p]
     L.fa_mlp_classify_features.argtypes = [H, H, C.c_int64, C.c_void_p, C.c_size_t]
+    L.fa_mlp_train.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_void_p,
+                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(FaTrainOpts), C.c_int,
+                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_char_p, C.c_size_t]
     L.fa_copy_peak_candidates.argtypes = [H, C.c_int64, C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_int32)]
     L.fa_hop_samples.argtypes = [cfgp, C.c_int]
     L.fa_frames_for.argtypes = [cfgp, C.c_int, C.c_size_t]

@@ -59,3 +59,7 @@ class FaCounts(C.Structure):
                 ("bands", C.c_int32), ("segments", C.c_int32), ("stored_segments", C.c_int32),
                 ("formant_rows", C.c_int32), ("syllables", C.c_int32), ("feature_rows", C.c_int32),
                 ("overflow", C.c_int32)]
+
+
+class FaTrainOpts(C.Structure):
+    _fields_ = [("learning_rate", C.c_double), ("optimizer", C.c_int32), ("epochs", C.c_int32), ("batch_size", C.c_int32)]

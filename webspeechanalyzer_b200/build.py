@@ -15,9 +15,9 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libfa_b200.so")
 SYNTH_LIB = os.path.join(HERE, "libfa_synth.so")   # host-only workload generator (bench / tests), not part of the product
-SOURCES = ["fa_spectrum.cu", "fa_peaks.cu", "fa_segment.cu", "fa_features.cu", "fa_utterance.cu", "fa_curves.cu", "fa_mlp.cu", "fa_capi.cu"]
+SOURCES = ["fa_spectrum.cu", "fa_peaks.cu", "fa_segment.cu", "fa_features.cu", "fa_utterance.cu", "fa_curves.cu", "fa_mlp.cu", "fa_train.cu", "fa_capi.cu"]
 HEADERS = [os.path.join(CSRC, "fa_internal.cuh")] + [os.path.join(ROOT, "include", h)
-                                                      for h in ("fa_b200.h", "fa_jsmath.h", "fa_tables.h", "fa_curves.h")]
+                                                      for h in ("fa_b200.h", "fa_jsmath.h", "fa_tables.h", "fa_curves.h", "fa_train.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "--fmad=false", "-std=c++17",
          "-Xcompiler", "-fPIC,-ffp-contract=off,-fvisibility=hidden", "-diag-suppress", "39,222",

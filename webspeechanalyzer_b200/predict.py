@@ -3,10 +3,12 @@
     reference                                                          here
     ml5.neuralNetwork(...).load(model.json, model_meta.json, weights)  load_tfjs_model(dir)  (tf.js layers format)
     nn.classifyMultiple(rows, cb)   src/neuralmodel.js:540-585          Classifier.classify_multiple(rows)
+    nn.train(...) + nn.save()       src/neuralmodel.js:163-403          train(rows, labels, ...) + save_tfjs_model(model, dir)
     predict_by_multiple_syllables / nn_prediction / seg_confidence_sort  SegmentVoter
                                     src/prediction.js:47-169
 
-The forward pass runs on the GPU (csrc/fa_mlp.cu behind fa_mlp_* of include/fa_b200.h); there is no CPU path.
+The forward pass runs on the GPU (csrc/fa_mlp.cu behind fa_mlp_* of include/fa_b200.h), and so does training (csrc/fa_train.cu
+behind fa_mlp_train; the algorithm is defined in DESIGN.md "K9"); there is no CPU path.
 Classifier.classify_features(engine) classifies the rows of a finished batch where they are -- in HBM.
 Model files are read at run time from a directory the caller names (e.g. dist/nnmodel/1/cats_emotion of the web app);
 nothing of the reference's models is stored in this repository."""
@@ -23,6 +25,10 @@ from . import _capi
 from ._capi import FaError
 
 ACTIVATIONS = {"linear": 0, "relu": 1, "sigmoid": 2, "softmax": 3}
+ACTIVATION_NAMES = {v: k for k, v in ACTIVATIONS.items()}
+OPTIMIZERS = {"sgd": 0, "adam": 1}
+# learning rate when the caller names none: ml5's classification SGD rate, tf.js's Adam default (INTEGRATION.md section 3)
+DEFAULT_LEARNING_RATE = {"sgd": 0.2, "adam": 0.001}
 
 
 def load_tfjs_model(model_dir: str, model_json: str = "model.json", meta_json: str = "model_meta.json") -> dict:
@@ -187,3 +193,142 @@ class SegmentVoter:
             if max_all > self.max_inv_entropy:
                 self.max_inv_entropy, self.min_entropy_db = max_all, d
         return top, best / seg_weight
+
+
+def save_tfjs_model(model: dict, model_dir: str) -> str:
+    """Write `model` (the dict load_tfjs_model returns) as the files ml5 saves: model.json (tf.js layers format, weights in
+    ./model.weights.bin), model.weights.bin and model_meta.json (normalised inputs with their ranges, the label legend)."""
+    os.makedirs(model_dir, exist_ok=True)
+    dims, labels = list(model["dims"]), list(model["labels"])
+    layers, specs, blob = [], [], b""
+    for i, (k, b, a) in enumerate(zip(model["kernels"], model["biases"], model["activations"])):
+        name = f"dense_Dense{i + 1}"
+        cfg = {"units": dims[i + 1], "activation": ACTIVATION_NAMES[int(a)], "use_bias": True, "name": name,
+               "kernel_initializer": {"class_name": "GlorotUniform", "config": {"seed": None}},
+               "bias_initializer": {"class_name": "Zeros", "config": {}}}
+        if i == 0:
+            cfg["batch_input_shape"] = [None, dims[0]]
+        layers.append({"class_name": "Dense", "config": cfg})
+        specs += [{"name": name + "/kernel", "shape": [dims[i], dims[i + 1]], "dtype": "float32"},
+                  {"name": name + "/bias", "shape": [dims[i + 1]], "dtype": "float32"}]
+        blob += np.ascontiguousarray(k, "<f4").tobytes() + np.ascontiguousarray(b, "<f4").tobytes()
+    doc = {"modelTopology": {"class_name": "Sequential", "config": {"name": "sequential_1", "layers": layers},
+                             "keras_version": "tfjs-layers", "backend": "tensor_flow.js"},
+           "format": "layers-model", "weightsManifest": [{"paths": ["./model.weights.bin"], "weights": specs}]}
+    meta = {"inputUnits": [dims[0]], "outputUnits": dims[-1],
+            "inputs": {str(i): {"dtype": "number", "min": float(model["in_min"][i]), "max": float(model["in_max"][i])}
+                       for i in range(dims[0])},
+            "outputs": {"label": {"dtype": "string", "min": 0, "max": 1, "uniqueValues": labels,
+                                  "legend": {lab: [1 if j == i else 0 for j in range(len(labels))] for i, lab in enumerate(labels)}}},
+            "isNormalized": True}
+    with open(os.path.join(model_dir, "model.json"), "w") as f:
+        json.dump(doc, f)
+    with open(os.path.join(model_dir, "model_meta.json"), "w") as f:
+        json.dump(meta, f)
+    with open(os.path.join(model_dir, "model.weights.bin"), "wb") as f:
+        f.write(blob)
+    return model_dir
+
+
+def row_labels(engine, utt_labels) -> np.ndarray:
+    """The app's "label from the file name" flow: utt_labels[u] (one per utterance of a finished Engine batch, in submission
+    order) repeated over that utterance's feature rows, aligned with engine.feature_table()."""
+    counts = engine.counts_table()["feature_rows"]
+    utt_labels = np.asarray(utt_labels)
+    if utt_labels.shape[0] != counts.shape[0]:
+        raise ValueError(f"{utt_labels.shape[0]} labels for {counts.shape[0]} utterances")
+    return np.repeat(utt_labels, counts)
+
+
+def glorot_params(dims, seed: int) -> np.ndarray:
+    """tf.js Dense defaults in K7's flat layout: per layer a Glorot-uniform kernel [in][out] (limit sqrt(6 / (in + out))),
+    then a zero bias; drawn from numpy.random.default_rng(seed), layer after layer."""
+    rng = np.random.default_rng(seed)
+    parts = []
+    for a, b in zip(dims[:-1], dims[1:]):
+        lim = math.sqrt(6.0 / (a + b))
+        parts += [rng.uniform(-lim, lim, (a, b)).astype(np.float32).ravel(), np.zeros(b, np.float32)]
+    return np.concatenate(parts)
+
+
+def _flat_params(model: dict) -> np.ndarray:
+    parts = []
+    for k, b in zip(model["kernels"], model["biases"]):
+        parts += [np.asarray(k, np.float32).ravel(), np.asarray(b, np.float32).ravel()]
+    return np.concatenate(parts)
+
+
+def train(rows, labels, label_names, hidden=(256, 64, 16), activations="relu", optimizer: str = "adam",
+          learning_rate: float | None = None, epochs: int = 32, batch_size: int = 32, seed=0, jobs=None, init: dict | None = None,
+          device: int = 0):
+    """Train a classifier of feature rows on the GPU (K9; one launch for all jobs and epochs).
+
+    rows [n, d] (float64), labels [n] (int indices into label_names).  The model is d -> hidden... -> len(label_names)
+    softmax, hidden layers with `activations` (one name, or one per hidden layer); with `init` (a model dict, e.g. from
+    load_tfjs_model) the architecture, start weights and input ranges are init's instead (fine-tuning).  optimizer "sgd" or
+    "adam"; learning_rate None takes DEFAULT_LEARNING_RATE[optimizer].  jobs None: one job on all rows, and one model is
+    returned; otherwise a list of row-index arrays (repeats oversample, disjoint lists give folds) and a list of models,
+    one per job.  seed: an int (job j uses seed + j: start weights and batch order) or one int per job.
+    Each model is the dict load_tfjs_model returns (Classifier and save_tfjs_model take it as it is) plus
+    "history": {"loss": [epochs], "accuracy": [epochs]}."""
+    rows = np.ascontiguousarray(rows, np.float64)
+    if rows.ndim != 2:
+        raise ValueError("rows must be [n, d]")
+    labels = np.ascontiguousarray(labels, np.int32).reshape(-1)
+    if labels.shape[0] != rows.shape[0]:
+        raise ValueError(f"{labels.shape[0]} labels for {rows.shape[0]} rows")
+    label_names = [str(x) for x in label_names]
+    if init is not None:
+        dims, acts = [int(x) for x in init["dims"]], [int(x) for x in init["activations"]]
+        if dims[0] != rows.shape[1] or dims[-1] != len(label_names):
+            raise ValueError(f"init is {dims[0]} -> {dims[-1]}, the data {rows.shape[1]} -> {len(label_names)}")
+    else:
+        dims = [rows.shape[1], *[int(h) for h in hidden], len(label_names)]
+        hid = [activations] * len(hidden) if isinstance(activations, str) else list(activations)
+        if len(hid) != len(hidden):
+            raise ValueError("one activation per hidden layer")
+        acts = [ACTIVATIONS[a] for a in hid] + [ACTIVATIONS["softmax"]]
+    if optimizer not in OPTIMIZERS:
+        raise ValueError(f"optimizer must be one of {sorted(OPTIMIZERS)}")
+    lr = DEFAULT_LEARNING_RATE[optimizer] if learning_rate is None else float(learning_rate)
+    single = jobs is None
+    job_lists = [np.arange(rows.shape[0], dtype=np.int32)] if single else [np.asarray(x, np.int32).reshape(-1) for x in jobs]
+    n_jobs = len(job_lists)
+    seeds = [int(seed) + j for j in range(n_jobs)] if np.isscalar(seed) else [int(s) for s in seed]
+    if len(seeds) != n_jobs:
+        raise ValueError(f"{len(seeds)} seeds for {n_jobs} jobs")
+    offsets = np.zeros(n_jobs + 1, np.int64)
+    offsets[1:] = np.cumsum([len(x) for x in job_lists])
+    row_idx = np.ascontiguousarray(np.concatenate(job_lists) if n_jobs else np.zeros(0, np.int32), np.int32)
+    if init is not None:
+        init_params = np.tile(_flat_params(init), n_jobs)
+        ranges = np.tile(np.concatenate([np.asarray(init["in_min"], np.float64), np.asarray(init["in_max"], np.float64)]), n_jobs)
+    else:
+        init_params = np.concatenate([glorot_params(dims, s) for s in seeds]) if n_jobs else np.zeros(0, np.float32)
+        ranges = None
+    n_params = sum(a * b + b for a, b in zip(dims[:-1], dims[1:]))
+    nl = len(dims) - 1
+    opts = _capi.FaTrainOpts(learning_rate=lr, optimizer=OPTIMIZERS[optimizer], epochs=int(epochs), batch_size=int(batch_size))
+    out_params = np.empty(max(n_jobs, 1) * n_params, np.float32)
+    out_ranges = np.empty((max(n_jobs, 1), 2, dims[0]), np.float64)
+    history = np.empty((max(n_jobs, 1), max(int(epochs), 1), 2), np.float64)
+    err = C.create_string_buffer(512)
+    L = _capi.lib()
+    seeds_a = np.asarray(seeds, np.uint64)
+    rc = L.fa_mlp_train(nl, (C.c_int * (nl + 1))(*dims), (C.c_int * nl)(*acts), rows.ctypes.data, rows.shape[0],
+                        labels.ctypes.data, n_jobs, offsets.ctypes.data, row_idx.ctypes.data, seeds_a.ctypes.data,
+                        init_params.ctypes.data, None if ranges is None else ranges.ctypes.data, C.byref(opts), device,
+                        out_params.ctypes.data, out_ranges.ctypes.data, history.ctypes.data, err, len(err))
+    if rc != 0:
+        raise FaError(rc, err.value.decode() or L.fa_status_string(rc).decode())
+    models = []
+    for j in range(n_jobs):
+        flat, off = out_params[j * n_params: (j + 1) * n_params], 0
+        kernels, biases = [], []
+        for a, b in zip(dims[:-1], dims[1:]):
+            kernels.append(flat[off: off + a * b].reshape(a, b).copy()); off += a * b
+            biases.append(flat[off: off + b].copy()); off += b
+        models.append(dict(dims=list(dims), activations=list(acts), kernels=kernels, biases=biases,
+                           in_min=out_ranges[j, 0].copy(), in_max=out_ranges[j, 1].copy(), labels=list(label_names),
+                           history={"loss": history[j, :epochs, 0].copy(), "accuracy": history[j, :epochs, 1].copy()}))
+    return models[0] if single else models
