@@ -297,8 +297,11 @@ FA_API int fa_copy_curve_features(fa_handle* h, int64_t utt_id, double* dst, siz
  * inputs are min-max normalised with the ranges of model_meta.json ((x - min) / (max - min), in double, then float32).
  * fa_mlp_classify takes host rows (n_rows x dims[0] doubles) and writes n_rows x dims[n_layers] float32 outputs;
  * fa_mlp_classify_features classifies the feature rows of a finished handle where they are (device), one utterance
- * (utt_id >= 0) or the whole batch (utt_id < 0), and returns the number of rows.  No CPU path: FA_ERR_NO_DEVICE without a B200. */
+ * (utt_id >= 0) or the whole batch (utt_id < 0), and returns the number of rows.  No CPU path: FA_ERR_NO_DEVICE without a B200.
+ * Every width dims[l], the input included, is at most FA_MLP_MAX_UNITS (the activations of K7's 8-row tile, two buffers of
+ * 8 x 3200 floats, take 200 KB of shared memory); fa_mlp_create returns FA_ERR_UNSUPPORTED for a wider model. */
 #define FA_MLP_MAX_LAYERS 8
+#define FA_MLP_MAX_UNITS 3200
 #define FA_MLP_LINEAR 0
 #define FA_MLP_RELU 1
 #define FA_MLP_SIGMOID 2
@@ -317,11 +320,12 @@ FA_API int fa_mlp_classify_features(fa_mlp* m, fa_handle* h, int64_t utt_id, flo
  * (n_rows x dims[0] doubles), its `labels` (int32 in [0, dims[n_layers])) and the options; job j trains on the row indices
  * row_idx[job_offsets[j] .. job_offsets[j + 1]) (repeats oversample, disjoint lists give folds), from its own seed and
  * initial parameters.  Parameter layout (init_params, out_params): per job, K7's -- for each layer the kernel [in][out],
- * then the bias, float32.  in_ranges NULL: each job's input ranges are the min / max of its own rows (a constant column
- * gets max = min + 1); otherwise [n_jobs][2][dims[0]] (min row, then max row) used as given.  out_ranges has that shape,
- * out_history is [n_jobs][epochs][2]: the row-weighted mean loss and the arg-max accuracy of every epoch.  Returns FA_OK,
- * FA_ERR_INVALID_ARG with a message in err (labels, indices, empty jobs, options, non-softmax output, non-finite values in
- * a selected row), FA_ERR_NO_DEVICE without an sm_100 device, or FA_ERR_CUDA / FA_ERR_OUT_OF_MEMORY. */
+ * then the bias, float32.  Widths are those fa_mlp_create accepts, every dims[l] in [1, FA_MLP_MAX_UNITS], so that each
+ * trained model loads for inference.  in_ranges NULL: each job's input ranges are the min / max of its own rows (a constant
+ * column gets max = min + 1); otherwise [n_jobs][2][dims[0]] (min row, then max row) used as given.  out_ranges has that
+ * shape, out_history is [n_jobs][epochs][2]: the row-weighted mean loss and the arg-max accuracy of every epoch.  Returns
+ * FA_OK, FA_ERR_INVALID_ARG with a message in err (widths, labels, indices, empty jobs, options, non-softmax output, non-finite
+ * values in a selected row), FA_ERR_NO_DEVICE without an sm_100 device, or FA_ERR_CUDA / FA_ERR_OUT_OF_MEMORY. */
 #define FA_OPT_SGD 0
 #define FA_OPT_ADAM 1 /* beta1 0.9, beta2 0.999, epsilon 1e-7, bias-corrected (tf.js defaults) */
 typedef struct fa_train_opts {

@@ -1,5 +1,6 @@
 /*
- * fa_train.h -- the seeded batch order of K9 (csrc/fa_train.cu), shared by the kernel and anything that restates it.
+ * fa_train.h -- the seeded batch order and the launch geometry of K9 (csrc/fa_train.cu), shared by the kernel and
+ * anything that restates them.
  *
  * Epoch e of a job with seed s visits its row list in the order row_idx[fa_perm(i, n, s, e)], i = 0 .. n - 1.
  * fa_perm is a bijection of [0, n): a 4-round balanced Feistel network on 2h bits (2^(2h) >= n, h >= 1), keyed by
@@ -12,11 +13,63 @@
 
 #include <stdint.h>
 
+#include "fa_b200.h"
+
 #if defined(__CUDACC__)
 #define FA_TRAIN_FN static inline __host__ __device__
 #else
 #define FA_TRAIN_FN static inline
 #endif
+
+#define FA_TRAIN_THREADS 512 /* threads of the CTA that trains one job */
+#define FA_TRAIN_TILE 8      /* rows per thread in the forward and delta phases; the batch is padded to a multiple */
+
+/* Where one fa_mlp_train launch keeps what.  Dynamic shared memory starts with red ([2][FA_TRAIN_THREADS] doubles, the
+ * partial min / max of the range reduction) and rng ([2][dims[0]] doubles, the ranges).  Then comes the batch area when
+ * it fits under the shared-memory cap; otherwise each job has a slice of area_bytes in global scratch.  The batch area
+ * holds the per-row tables (loss: double[bpad]; row, label, hit: int[bpad] each) and, from act_off, the activations.
+ * Offsets in floats (parameters, activations) or bytes (the rest); every size is 64-bit. */
+typedef struct fa_train_geom {
+  int64_t bpad;                               /* the batch size rounded up to FA_TRAIN_TILE rows */
+  int64_t w_off[FA_MLP_MAX_LAYERS];           /* floats: kernel [dims[l]][dims[l + 1]] of layer l (K7's layout) */
+  int64_t b_off[FA_MLP_MAX_LAYERS];           /* floats: its bias */
+  int64_t n_params;                           /* floats of parameters per job */
+  int64_t a_off[FA_MLP_MAX_LAYERS + 1];       /* floats: activations (then deltas) [bpad][dims[l]] of layer l */
+  int64_t n_act;                              /* floats of activations per job */
+  int64_t act_off;                            /* bytes from the start of the batch area to the activations */
+  int64_t area_bytes;                         /* bytes of one job's batch area, a multiple of 16 */
+  int64_t area_smem_off;                      /* bytes from the start of dynamic shared memory to the batch area */
+  int area_in_smem;                           /* 1: the batch area is in shared memory; 0: per-job global scratch */
+  int64_t smem_bytes;                         /* dynamic shared memory of the launch */
+} fa_train_geom;
+
+/* The geometry of n_layers layers (dims[0 .. n_layers]) at batch size `batch`: the batch area goes to shared memory when
+ * the whole launch then needs at most smem_cap bytes.  Returns 0, or -1 when the launch cannot be served: more than
+ * smem_optin bytes of shared memory (the block's opt-in limit minus the kernel's static shared memory), or a parameter or
+ * activation count past the kernel's 32-bit indexing. */
+FA_TRAIN_FN int fa_train_geometry(const int* dims, int n_layers, int batch, int64_t smem_cap, int64_t smem_optin,
+                                  fa_train_geom* g) {
+  int64_t off = 0, act = 0;
+  g->bpad = ((int64_t)batch + FA_TRAIN_TILE - 1) / FA_TRAIN_TILE * FA_TRAIN_TILE;
+  for (int l = 0; l <= FA_MLP_MAX_LAYERS; l++) g->a_off[l] = 0;   /* entries past n_layers stay 0 */
+  for (int l = 0; l < FA_MLP_MAX_LAYERS; l++) g->w_off[l] = g->b_off[l] = 0;
+  for (int l = 0; l <= n_layers; l++) {
+    g->a_off[l] = act;
+    act += g->bpad * dims[l];
+  }
+  for (int l = 0; l < n_layers; l++) {
+    g->w_off[l] = off; off += (int64_t)dims[l] * dims[l + 1];
+    g->b_off[l] = off; off += dims[l + 1];
+  }
+  g->n_params = off;
+  g->n_act = act;
+  g->act_off = g->bpad * (int64_t)(sizeof(double) + 3 * sizeof(int32_t));
+  g->area_bytes = (g->act_off + act * (int64_t)sizeof(float) + 15) / 16 * 16;
+  g->area_smem_off = (2 * FA_TRAIN_THREADS + 2 * (int64_t)dims[0]) * (int64_t)sizeof(double);
+  g->area_in_smem = g->area_smem_off + g->area_bytes <= smem_cap;
+  g->smem_bytes = g->area_smem_off + (g->area_in_smem ? g->area_bytes : 0);
+  return g->smem_bytes <= smem_optin && g->n_params <= INT32_MAX && g->n_act <= INT32_MAX ? 0 : -1;
+}
 
 #define FA_PERM_ROUNDS 4
 

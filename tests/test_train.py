@@ -1,9 +1,10 @@
 """Training of the feature-row classifier (K9, csrc/fa_train.cu; algorithm in DESIGN.md "K9").
 
 CPU: the model writer round-trips through the loader, the numpy restatement of the batch order is a bijection, the options
-struct matches the header, host-side rejections, and no CPU fallback.  GPU: SGD and Adam against this file's own float64
-trainer of the same algorithm (same start values, order and ranges), determinism and job independence, learning,
-fine-tune passthrough, real rows from an Engine and the device-side rejection of non-finite rows."""
+struct matches the header, the launch geometry fits every accepted input, host-side rejections, and no CPU fallback.
+GPU: SGD and Adam against this file's own float64 trainer of the same algorithm (same start values, order and ranges) --
+on the default shape and on a table of cases that takes every branch of the kernel -- determinism and job independence,
+learning, fine-tune passthrough, real rows from an Engine and the device-side rejection of non-finite rows."""
 import ctypes as C
 import json
 import os
@@ -121,14 +122,16 @@ def train_f64(rows, labels, dims, acts, flat, lo, hi, idx, seed, epochs, batch, 
     return Ws, bs, hist, grads_log
 
 
-def four_class(n, seed, spread=1.0, d=53):
-    """Seeded 4-class rows: class centres in a 53-dim space with per-column scales and offsets; column 5 is constant."""
+def four_class(n, seed, spread=1.0, d=53, k=4):
+    """Seeded rows of k classes (4 by default): class centres in a d-dim space with per-column scales and offsets; column 5
+    (if there is one) is constant."""
     rng = np.random.default_rng(seed)
-    centres = rng.normal(0, 1, (4, d))
-    y = rng.integers(0, 4, n).astype(np.int32)
+    centres = rng.normal(0, 1, (k, d))
+    y = rng.integers(0, k, n).astype(np.int32)
     x = centres[y] + spread * rng.normal(0, 1, (n, d))
     x = x * rng.uniform(0.5, 200, d) + rng.uniform(-50, 50, d)
-    x[:, 5] = 3.25
+    if d > 5:
+        x[:, 5] = 3.25
     return x, y
 
 
@@ -208,6 +211,72 @@ def test_options_struct_matches_the_header(tmp_path):
     assert got == want and [f for f, _ in T._fields_] == ["learning_rate", "optimizer", "epochs", "batch_size"]
 
 
+GEOMETRY_C = r"""#include <stdio.h>
+#include <stdlib.h>
+#include "fa_train.h"
+int main(int argc, char** argv) {   /* batch smem_optin dims[0] .. dims[n_layers] */
+  int dims[FA_MLP_MAX_LAYERS + 1], n_layers = argc - 4;
+  for (int l = 0; l <= n_layers; l++) dims[l] = atoi(argv[3 + l]);
+  fa_train_geom g;
+  int rc = fa_train_geometry(dims, n_layers, atoi(argv[1]), 200 * 1024, atoll(argv[2]), &g);
+  printf("%d %lld %lld %lld %lld %lld %lld %d %lld", rc, (long long)g.bpad, (long long)g.n_params, (long long)g.n_act,
+         (long long)g.act_off, (long long)g.area_bytes, (long long)g.area_smem_off, g.area_in_smem, (long long)g.smem_bytes);
+  for (int l = 0; l <= n_layers; l++) printf(" %lld", (long long)g.a_off[l]);
+  for (int l = 0; l < n_layers; l++) printf(" %lld %lld", (long long)g.w_off[l], (long long)g.b_off[l]);
+  printf("\n");
+  return 0;
+}
+"""
+SMEM_OPTIN = 227 * 1024 - 16      # a B200 block's opt-in shared memory minus fa_train_kernel's 16 bytes of static shared memory
+
+
+def geometry_py(dims, batch, cap=200 * 1024):
+    """DESIGN.md "K9" / include/fa_train.h restated: red + rng, then the batch area (per-row tables: 8 + 3 x 4 bytes a
+    row; activations) in shared memory when the launch stays under `cap`, else in per-job global scratch."""
+    bpad = -(-batch // 8) * 8
+    a_off = [bpad * sum(dims[:l]) for l in range(len(dims))]
+    wb, off = [], 0
+    for a, b in zip(dims[:-1], dims[1:]):
+        wb += [off, off + a * b]
+        off += a * b + b
+    n_act = bpad * sum(dims)
+    act_off = 20 * bpad
+    area = -(-(act_off + 4 * n_act) // 16) * 16
+    area_smem_off = 8 * (2 * 512 + 2 * dims[0])
+    in_smem = int(area_smem_off + area <= cap)
+    return [0, bpad, off, n_act, act_off, area, area_smem_off, in_smem, area_smem_off + (area if in_smem else 0)] + a_off + wb
+
+
+@pytest.mark.parametrize("dims, batch, in_smem", [
+    ((53, 256, 64, 16, 4), 32, 1),          # the default shape: 59 984 B of shared memory
+    ((53, 256, 64, 16, 4), 256, 0),         # activations past the 200 KB cap
+    ((53, 48, 24, 12, 5), 20, 1),           # padding rows
+    ((1, 4, 2), 1, 1),
+    ((53, 8, 4), 11170, 0),                 # per-row tables in shared memory would pass 227 KB here
+    ((53, 8, 4), 12000, 0),
+    ((53, 8, 4), 65536, 0),                 # the largest batch
+    ((3200, 64, 4), 8700, 0),               # the widest input: 50 KB of ranges
+    ((3200,) * 9, 65536, 0),                # the largest model the host accepts
+], ids=lambda v: "-".join(map(str, v)) if isinstance(v, tuple) else str(v))
+def test_launch_geometry_fits_every_accepted_input(tmp_path, dims, batch, in_smem):
+    """fa_train_geometry (include/fa_train.h, what fa_mlp_train launches with): every input the host accepts fits the
+    block's shared memory, its activation offsets fit the kernel's 32-bit indexing, and the layout is the restated one."""
+    src = tmp_path / "geom.c"
+    src.write_text(GEOMETRY_C)
+    exe = str(tmp_path / "geom")
+    subprocess.check_call(["gcc", "-std=c99", "-Wall", "-Werror", "-I", os.path.join(ROOT, "include"), "-o", exe, str(src)])
+
+    def run(optin):
+        return [int(v) for v in subprocess.check_output([exe, str(batch), str(optin), *map(str, dims)], text=True).split()]
+    got = run(SMEM_OPTIN)
+    assert got == geometry_py(dims, batch)
+    rc, n_act, in_smem_got, smem = got[0], got[3], got[7], got[8]
+    assert rc == 0 and in_smem_got == in_smem and smem <= SMEM_OPTIN and n_act <= 2**31 - 1
+    assert run(smem)[0] == 0 and run(smem - 1)[0] == -1
+    if dims == (53, 256, 64, 16, 4) and batch == 32:
+        assert smem == 59984
+
+
 def expect_invalid(match, *args, **kw):
     with pytest.raises(FaError) as e:
         predict.train(*args, **kw)
@@ -231,6 +300,11 @@ def test_rejections_on_the_host(tmp_path):
     expect_invalid("output activation must be softmax", x, y, names, init=init, epochs=1)
     init = predict.load_tfjs_model(write_model(str(tmp_path / "b"), acts=("softmax", "relu", "relu", "softmax")))
     expect_invalid("hidden layer 0", x, y, names, init=init, epochs=1)
+    # FA_MLP_MAX_UNITS: a wider layer, or a wider input, would train and then not load into Classifier
+    expect_invalid("dims[1] must be in [1, 3200]", x, y, names, hidden=(3201,), epochs=1)
+    expect_invalid("dims[2] must be in [1, 3200]", x, y, names, hidden=(16, 4000), epochs=1)
+    wide, wy = four_class(20, 2, d=3201)
+    expect_invalid("dims[0] must be in [1, 3200]", wide, wy, names, hidden=(8,), epochs=1)
 
 
 NO_DEVICE_CHECK = """
@@ -263,6 +337,18 @@ def layer_close(got, Ws, bs, tol=1e-4, exempt=None):
             assert d.max() <= tol * scale, (l, i, d.max(), scale)
 
 
+def adam_exempt(grads):
+    """Masks of the parameters whose gradient was near zero at some step: its sign decides +-lr in m / sqrt(v)."""
+    nl = len(grads[0]) // 2
+    exempt = [np.zeros(g.shape, bool) for g in grads[0]]
+    for gs in grads:
+        for l in range(nl):
+            big = max(np.abs(gs[l]).max(), np.abs(gs[l + nl]).max())
+            exempt[l] |= np.abs(gs[l]) < 1e-6 * big
+            exempt[l + nl] |= np.abs(gs[l + nl]) < 1e-6 * big
+    return exempt
+
+
 @pytest.mark.gpu
 def test_sgd_matches_float64():
     x, y = four_class(2000, 11)
@@ -289,19 +375,180 @@ def test_adam_matches_float64():
     m = predict.train(x, y, names, optimizer="adam", learning_rate=1e-3, epochs=1, jobs=[idx], seed=[4])[0]
     Ws, bs, _, grads = train_f64(x, y, dims, acts, predict.glorot_params(dims, 4), lo, hi, idx, 4, 1, 32, "adam", 1e-3)
     assert len(grads) == 5
-    nl = len(Ws)
-    exempt = [np.zeros(g.shape, bool) for g in grads[0]]
-    for gs in grads:                   # a near-zero gradient's sign decides +-lr in m / sqrt(v)
-        for l in range(nl):
-            big = max(np.abs(gs[l]).max(), np.abs(gs[l + nl]).max())
-            exempt[l] |= np.abs(gs[l]) < 1e-6 * big
-            exempt[l + nl] |= np.abs(gs[l + nl]) < 1e-6 * big
-    layer_close(m, Ws, bs, exempt=exempt)
+    layer_close(m, Ws, bs, exempt=adam_exempt(grads))
     m5 = predict.train(x, y, names, optimizer="adam", learning_rate=1e-3, epochs=5, seed=5)
     _, _, hist, _ = train_f64(x, y, dims, acts, predict.glorot_params(dims, 5), *job_ranges(x, np.arange(2000)),
                               np.arange(2000), 5, 5, 32, "adam", 1e-3)
     ref = np.array(hist)[:, 0]
     assert np.all(np.abs(m5["history"]["loss"] - ref) <= 1e-3 * ref)
+
+
+# ---- every path of the kernel against the float64 trainer, each run a few dozen steps at most -------------------------
+NAMES4 = ["N", "A", "S", "H"]
+
+
+def flat_of(m):
+    return np.concatenate([np.asarray(a, np.float32).ravel() for k, b in zip(m["kernels"], m["biases"]) for a in (k, b)])
+
+
+def train_and_check(x, y, names, jobs, seeds, hidden=(), acts="relu", optimizer="sgd", lr=0.1, epochs=1, batch=32, init=None):
+    """predict.train on `jobs`, then every job against train_f64 from the same start values, order and ranges: parameters
+    within 1e-4 of the layer's largest |w| (Adam: but for near-zero gradients), per-epoch loss within 1e-5 (SGD) or 1e-3
+    (Adam) relative, accuracy within 2 rows, ranges bit-equal; and K7 scores every model within 1e-5 of forward_f32."""
+    models = predict.train(x, y, names, hidden=hidden, activations=acts, optimizer=optimizer, learning_rate=lr,
+                           epochs=epochs, batch_size=batch, jobs=jobs, seed=seeds, init=init)
+    for m, idx, seed in zip(models, jobs, seeds):
+        idx = np.asarray(idx)
+        if init is None:
+            lo, hi = job_ranges(x, idx)
+            flat = predict.glorot_params(m["dims"], seed)
+        else:
+            lo, hi = np.asarray(init["in_min"], np.float64), np.asarray(init["in_max"], np.float64)
+            flat = flat_of(init)
+        assert m["in_min"].tobytes() == lo.tobytes() and m["in_max"].tobytes() == hi.tobytes()
+        Ws, bs, hist, grads = train_f64(x, y, m["dims"], m["activations"], flat, lo, hi, idx, seed, epochs, batch, optimizer, lr)
+        layer_close(m, Ws, bs, exempt=adam_exempt(grads) if optimizer == "adam" else None)
+        ref = np.array(hist)
+        rel = 1e-5 if optimizer == "sgd" else 1e-3
+        assert np.all(np.abs(m["history"]["loss"] - ref[:, 0]) <= rel * ref[:, 0]), (m["history"]["loss"], ref[:, 0])
+        assert np.all(np.abs(m["history"]["accuracy"] - ref[:, 1]) <= 2 / len(idx))
+        rows = x[idx[:1024]]
+        clf = predict.Classifier(m)
+        assert np.abs(clf.probabilities(rows) - forward_f32(m, rows)).max() <= 1e-5
+        clf.close()
+    return models
+
+
+def case_sigmoid():
+    x, y = four_class(1000, 21)
+    for opt, lr in (("sgd", 0.5), ("adam", 1e-3)):
+        train_and_check(x, y, NAMES4, [np.arange(1000)], [7], hidden=(64, 16), acts="sigmoid", optimizer=opt, lr=lr)
+
+
+def case_mixed():
+    """linear backward, 5 classes, 4 padding rows per batch of 20, a last batch of 17"""
+    x, y = four_class(517, 22, k=5)
+    train_and_check(x, y, list("abcde"), [np.arange(517)], [8], hidden=(48, 24, 12), acts=["linear", "sigmoid", "relu"],
+                    lr=0.2, batch=20)
+
+
+def case_no_hidden():
+    """one layer (no delta phase), one padding row per batch of 7"""
+    x, y = four_class(300, 23, k=3)
+    train_and_check(x, y, list("abc"), [np.arange(300)], [9], lr=0.5, batch=7)
+
+
+def case_deep():
+    x, y = four_class(320, 24)
+    train_and_check(x, y, NAMES4, [np.arange(320)], [10], hidden=(32,) * 7, acts=["relu", "sigmoid"] * 3 + ["relu"],
+                    lr=0.5, batch=16)
+
+
+def case_wide():
+    """widths above the 512 threads of a job and not a multiple of 32, 2 classes"""
+    x, y = four_class(200, 25, k=2)
+    train_and_check(x, y, ["x", "y"], [np.arange(200)], [11], hidden=(600, 37), lr=0.1, batch=8)
+
+
+def case_inputs():
+    """the range reduction over 1, 2 and 3 chunks of 512 columns, constant columns in the first and the last chunk"""
+    x, y = four_class(300, 26, d=1, k=2)
+    train_and_check(x, y, ["x", "y"], [np.arange(300)], [12], hidden=(4,), lr=0.5)
+    for d in (600, 1030):
+        x, y = four_class(400, 27, d=d)
+        x[:, d - 1] = -7.5
+        train_and_check(x, y, NAMES4, [np.arange(13, 269)], [13], hidden=(16,), lr=0.1)
+
+
+def case_batch_edges():
+    x, y = four_class(200, 28)
+    train_and_check(x, y, NAMES4, [np.arange(40)], [14], hidden=(16,), lr=0.1, batch=1)
+    train_and_check(x, y, NAMES4, [np.arange(100, 145)], [15], hidden=(16,), optimizer="adam", lr=1e-3, epochs=3, batch=64)
+
+
+def case_global_scratch():
+    """the default shape at batch 256: per-row tables and activations in per-job slices of global scratch"""
+    x, y = four_class(1500, 29)
+    rng = np.random.default_rng(3)
+    jobs = [rng.choice(1500, 300, replace=False), rng.choice(1500, 700, replace=True), np.arange(200, 720)]
+    seeds = [31, 32, 33]
+    together = train_and_check(x, y, NAMES4, jobs, seeds, hidden=(256, 64, 16), lr=0.1, epochs=2, batch=256)
+    for j in range(3):
+        alone = predict.train(x, y, NAMES4, hidden=(256, 64, 16), optimizer="sgd", learning_rate=0.1, epochs=2,
+                              batch_size=256, jobs=[jobs[j]], seed=[seeds[j]])[0]
+        assert_same_model(model_of(together[j]), model_of(alone))
+        assert together[j]["history"]["loss"].tobytes() == alone["history"]["loss"].tobytes()
+
+
+def case_big_batch():
+    """batches whose per-row tables alone exceed a block's shared memory, up to the largest batch accepted"""
+    x, y = four_class(66536, 30)
+    train_and_check(x, y, NAMES4, [np.arange(30000)], [16], hidden=(8,), lr=0.5, batch=12000)
+    train_and_check(x, y, NAMES4, [np.arange(66536)], [17], hidden=(8,), lr=0.5, batch=65536)
+
+
+def case_fine_tune():
+    """shipped model 1 as the start, its ranges as given, and rows outside them (normalised below 0 and above 1)"""
+    sys.path.insert(0, GOLDEN)
+    import npzparts
+    z = npzparts.load(os.path.join(GOLDEN, "mlp_shipped"))
+    mi = json.load(open(os.path.join(GOLDEN, "mlp_shipped.json")))["models"]["1"]
+    n = len(mi["dims"]) - 1
+    init = dict(dims=mi["dims"], activations=mi["activations"], kernels=[z[f"m1_k{i}"] for i in range(n)],
+                biases=[z[f"m1_b{i}"] for i in range(n)], in_min=z["m1_min"], in_max=z["m1_max"], labels=mi["labels"])
+    lo, hi = np.asarray(z["m1_min"], np.float64), np.asarray(z["m1_max"], np.float64)
+    rng = np.random.default_rng(4)
+    out = np.array(z["rows"][:25], np.float64)
+    up, down = np.split(rng.choice(53, 20, replace=False), 2)
+    out[:, up] = hi[up] + (hi - lo)[up] * rng.uniform(0.1, 0.5, (25, 10))
+    out[:, down] = lo[down] - (hi - lo)[down] * rng.uniform(0.1, 0.5, (25, 10))
+    x = np.vstack([z["rows"], out])
+    y = rng.integers(0, 4, x.shape[0]).astype(np.int32)
+    for opt, lr in (("sgd", 0.05), ("adam", 1e-3)):
+        train_and_check(x, y, mi["labels"], [np.arange(x.shape[0])], [18], optimizer=opt, lr=lr, epochs=2, batch=8, init=init)
+
+
+def case_jobs():
+    """repeated and disjoint row lists of different sizes and seeds; Adam's bias correction runs on across epochs"""
+    x, y = four_class(600, 31)
+    rng = np.random.default_rng(5)
+    p = rng.permutation(600)
+    jobs = [rng.choice(600, 96, replace=True), p[:40], p[40:110], np.repeat(p[110:129], 3)]
+    train_and_check(x, y, NAMES4, jobs, [41, 42, 43, 44], hidden=(64, 16), optimizer="adam", lr=1e-3, epochs=3)
+
+
+def case_zero_epochs():
+    x, y = four_class(300, 32)
+    idx = np.arange(50, 250)
+    lo, hi = job_ranges(x, idx)
+    for opt in ("sgd", "adam"):
+        m = predict.train(x, y, NAMES4, hidden=(64, 16), optimizer=opt, epochs=0, jobs=[idx], seed=[19])[0]
+        assert flat_of(m).tobytes() == predict.glorot_params(m["dims"], 19).tobytes()
+        assert m["in_min"].tobytes() == lo.tobytes() and m["in_max"].tobytes() == hi.tobytes()
+        assert m["history"]["loss"].shape == m["history"]["accuracy"].shape == (0,)
+
+
+def case_width_limit():
+    """FA_MLP_MAX_UNITS: K9's widest layer (activations in global scratch) loads into K7 (parameters read from global
+    memory, activations at its 200 KB cap); one unit more is refused by K7 (and by K9 on the host)"""
+    x, y = four_class(64, 33)
+    m = train_and_check(x, y, NAMES4, [np.arange(64)], [20], hidden=(3200,), lr=0.1)[0]
+    wider = dict(model_of(m), dims=[53, 3201, 4], kernels=[np.zeros((53, 3201), np.float32), np.zeros((3201, 4), np.float32)],
+                 biases=[np.zeros(3201, np.float32), np.zeros(4, np.float32)])
+    with pytest.raises(FaError) as e:
+        predict.Classifier(wider)
+    assert e.value.status == _capi.FA_ERR_UNSUPPORTED
+
+
+TRAIN_CASES = {f.__name__[5:]: f for f in (case_sigmoid, case_mixed, case_no_hidden, case_deep, case_wide, case_inputs,
+                                           case_batch_edges, case_global_scratch, case_big_batch, case_fine_tune,
+                                           case_jobs, case_zero_epochs, case_width_limit)}
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("case", list(TRAIN_CASES))
+def test_kernel_paths_match_float64(case):
+    TRAIN_CASES[case]()
 
 
 @pytest.mark.gpu

@@ -41,6 +41,8 @@ namespace {
 
 constexpr int kRowsPerCta = 8;
 constexpr int kMlpThreads = 256;
+// the activation buffers of the widest model fit the 200 KB that mlp_launch gives a CTA
+static_assert(2 * kRowsPerCta * FA_MLP_MAX_UNITS * sizeof(float) <= 200 * 1024, "FA_MLP_MAX_UNITS is past K7's activation buffers");
 
 struct MlpArgs {
   int n_layers;
@@ -191,7 +193,9 @@ int fa_mlp_create(int n_layers, const int* dims, const int* activations, const f
   m->device = device; m->n_layers = n_layers;
   int off = 0, mx = 0;
   for (int l = 0; l <= n_layers; l++) {
-    if (dims[l] < 1 || dims[l] > 4096) { delete m; return FA_ERR_INVALID_ARG; }
+    if (dims[l] < 1) { delete m; return FA_ERR_INVALID_ARG; }
+    // the activations of 8 rows must fit one CTA's shared memory; the parameters are staged there too when they fit (mlp_launch)
+    if (dims[l] > FA_MLP_MAX_UNITS) { delete m; return FA_ERR_UNSUPPORTED; }
     m->dims[l] = dims[l];
     mx = dims[l] > mx ? dims[l] : mx;
   }
@@ -202,8 +206,6 @@ int fa_mlp_create(int n_layers, const int* dims, const int* activations, const f
     m->b_off[l] = off; off += dims[l + 1];
   }
   m->n_params = off; m->max_dim = mx;
-  // the activations of 8 rows must fit one CTA's shared memory; the parameters are staged there too when they fit (mlp_launch)
-  if ((size_t)2 * kRowsPerCta * mx * sizeof(float) > 200 * 1024) { delete m; return FA_ERR_UNSUPPORTED; }
   std::vector<float> host((size_t)off);
   for (int l = 0; l < n_layers; l++) {
     memcpy(host.data() + m->w_off[l], kernels[l], sizeof(float) * (size_t)dims[l] * dims[l + 1]);

@@ -9,18 +9,18 @@
 // Mapping: one CTA of kTrainThreads threads per job, and one launch for the whole run -- a step is a few microseconds of
 // arithmetic with a strict dependency on the previous one, so the host never comes between steps.  Parameters, gradients
 // and Adam moments of a job live in global memory (they stay in L1 / L2: 124 KB for 53-256-64-16-4, 1.2 MB for
-// 53-512-512-8); the activations of a batch ([rows][dims[l]] per layer) live in shared memory when they fit and in a
-// per-job global scratch otherwise (same code, same order, same bits).  The backward sweep overwrites each layer's
-// activations with its deltas in place.  Per step: the batch's rows and inputs, one phase per layer forward (thread =
+// 53-512-512-8); the batch's per-row tables and activations ([rows][dims[l]] per layer) live in shared memory when they
+// fit and in a per-job global scratch otherwise (same code, same order, same bits; fa_train_geometry in
+// include/fa_train.h decides).  The backward sweep overwrites each layer's activations with its deltas in place.  Per step: the batch's rows and inputs, one phase per layer forward (thread =
 // output unit x 8 rows in registers), softmax / loss / output delta (thread = row), per layer a gradient phase
 // (thread = parameter, rows in order) and a delta phase (thread = input unit x 8 rows), then the optimizer over all
 // parameters; __syncthreads between phases.  float32 with explicit fmaf in a fixed index order (--fmad=false), loss and
 // accuracy summed by one thread in row order: a job's result depends on nothing but its own inputs.  Jobs fill the SMs.
 // No tensor cores: ~31 k MAC per row and step-to-step dependency, not FLOPs, bound the run.
 //
-// ptxas (sm_100a, -Xptxas -v, CUDA 12.9): fa_train_kernel 64 registers, 16 bytes static shared memory, 0 bytes stack,
-// 0 bytes spill stores / loads; dynamic shared memory 9.5 KB + the activations (50 KB for 53-256-64-16-4 at batch 32,
-// 139 KB for 53-512-512-8 at batch 32).
+// ptxas (sm_100a, -Xptxas -v, CUDA 12.9): fa_train_kernel 58 registers, 16 bytes static shared memory, 0 bytes stack,
+// 0 bytes spill stores / loads; dynamic shared memory 8 KB + 16 B per input column, then, when they fit, the per-row
+// tables (20 B per row) and the activations (50 KB for 53-256-64-16-4 at batch 32, 139 KB for 53-512-512-8 at batch 32).
 #include <climits>
 #include <cmath>
 #include <cstdio>
@@ -33,8 +33,8 @@
 
 namespace {
 
-constexpr int kTrainThreads = 512;
-constexpr int kTile = 8;                  // rows per thread in the forward and delta phases (register tile)
+constexpr int kTrainThreads = FA_TRAIN_THREADS;
+constexpr int kTile = FA_TRAIN_TILE;      // rows per thread in the forward and delta phases (register tile)
 constexpr int kSmemCap = 200 * 1024;      // dynamic shared memory a job may take
 constexpr float kBeta1 = 0.9f, kBeta2 = 0.999f, kOneMinusBeta1 = 0.1f, kOneMinusBeta2 = 0.001f, kEpsilon = 1e-7f;
 
@@ -44,7 +44,8 @@ struct TrainArgs {
   int act[FA_MLP_MAX_LAYERS];
   int w_off[FA_MLP_MAX_LAYERS], b_off[FA_MLP_MAX_LAYERS];
   int a_off[FA_MLP_MAX_LAYERS + 1];      // activations (then deltas) of layer l: [bpad][dims[l]] floats at a_off[l]
-  int n_params, n_act, act_smem_off;     // act_smem_off: byte offset of the activations in shared memory (act_g == nullptr)
+  int n_params, act_off, area_smem_off;  // bytes: activations in the batch area, the batch area in shared memory
+  size_t area_bytes;                     // bytes of one job's batch area (fa_train_geom)
   int batch, bpad, epochs, optimizer, given_ranges;
   float lr;
   const double* rows;                    // [n_rows][dims[0]]
@@ -55,7 +56,7 @@ struct TrainArgs {
   float* params;                         // [J][n_params]: start values in, trained values out
   float* grad;                           // [J][n_params]
   float* m1; float* m2;                  // [J][n_params] Adam moments (zero at the start), nullptr for SGD
-  float* act_g;                          // [J][n_act] when the activations do not fit shared memory, else nullptr
+  unsigned char* area_g;                 // [J][area_bytes] when the batch area does not fit shared memory, else nullptr
   double* ranges;                        // [J][2][dims[0]]: given ranges in (given_ranges), the ranges used out
   double* history;                       // [J][epochs][2]: mean loss, accuracy
   int* bad_row;                          // [J]: a table row with a non-finite value (INT_MAX: none)
@@ -68,11 +69,12 @@ __global__ void __launch_bounds__(kTrainThreads) fa_train_kernel(const TrainArgs
   const int L = a.n_layers, d0 = a.dims[0], nout = a.dims[L], bpad = a.bpad;
   double* red = reinterpret_cast<double*>(smem_raw);     // [2][kTrainThreads] partial min / max
   double* rng = red + 2 * kTrainThreads;                  // [2][d0] min, max
-  double* loss_r = rng + 2 * d0;                          // [bpad]
+  unsigned char* area = a.area_g ? a.area_g + (size_t)j * a.area_bytes : smem_raw + a.area_smem_off;
+  double* loss_r = reinterpret_cast<double*>(area);       // [bpad]
   int* rowid = reinterpret_cast<int*>(loss_r + bpad);     // [bpad]
   int* lab = rowid + bpad;
   int* hit_r = lab + bpad;
-  float* A = a.act_g ? a.act_g + (size_t)j * a.n_act : reinterpret_cast<float*>(smem_raw + a.act_smem_off);
+  float* A = reinterpret_cast<float*>(area + a.act_off);
   float* P = a.params + (size_t)j * a.n_params;
   float* G = a.grad + (size_t)j * a.n_params;
   float* M1 = a.m1 ? a.m1 + (size_t)j * a.n_params : nullptr;
@@ -310,8 +312,9 @@ extern "C" int fa_mlp_train(int n_layers, const int* dims, const int* activation
   if (!dims || !activations || !opts || !job_offsets || !row_idx || !seeds || !init_params || !out_params || !out_ranges ||
       (!out_history && opts->epochs > 0) || (n_rows && (!rows || !labels)))
     return fail(FA_ERR_INVALID_ARG, "null argument");
-  for (int l = 0; l <= n_layers; l++)
-    if (dims[l] < 1 || dims[l] > 4096) return fail(FA_ERR_INVALID_ARG, "dims[%lld] must be in [1, 4096]", l);
+  for (int l = 0; l <= n_layers; l++)   // every trained model loads into K7 (fa_mlp_create)
+    if (dims[l] < 1 || dims[l] > FA_MLP_MAX_UNITS)
+      return fail(FA_ERR_INVALID_ARG, "dims[%lld] must be in [1, %lld]", l, FA_MLP_MAX_UNITS);
   for (int l = 0; l + 1 < n_layers; l++)
     if (activations[l] != FA_MLP_LINEAR && activations[l] != FA_MLP_RELU && activations[l] != FA_MLP_SIGMOID)
       return fail(FA_ERR_INVALID_ARG, "hidden layer %lld: the activation must be linear, relu or sigmoid", l);
@@ -340,24 +343,30 @@ extern "C" int fa_mlp_train(int n_layers, const int* dims, const int* activation
   if (cudaGetDeviceProperties(&prop, device) != cudaSuccess || prop.major != 10)
     return fail(FA_ERR_NO_DEVICE, "not an sm_100 device");
   cudaSetDevice(device);
+  cudaFuncAttributes fattr;
+  if (cudaFuncGetAttributes(&fattr, fa_train_kernel) != cudaSuccess) return fail(FA_ERR_CUDA, "training kernel attributes");
+  fa_train_geom g;
+  if (fa_train_geometry(dims, n_layers, opts->batch_size, kSmemCap,
+                        (int64_t)prop.sharedMemPerBlockOptin - (int64_t)fattr.sharedSizeBytes, &g) != 0)
+    return fail(FA_ERR_UNSUPPORTED, "the training kernel cannot hold this model at batch_size %lld", opts->batch_size);
 
   TrainArgs a;
   memset(&a, 0, sizeof(a));
   a.n_layers = n_layers;
-  int off = 0, act_floats = 0;
-  a.bpad = (opts->batch_size + kTile - 1) / kTile * kTile;
+  a.bpad = (int)g.bpad;
   for (int l = 0; l <= n_layers; l++) {
     a.dims[l] = dims[l];
-    a.a_off[l] = act_floats;
-    act_floats += a.bpad * dims[l];
+    a.a_off[l] = (int)g.a_off[l];
   }
   for (int l = 0; l < n_layers; l++) {
     a.act[l] = activations[l];
-    a.w_off[l] = off; off += dims[l] * dims[l + 1];
-    a.b_off[l] = off; off += dims[l + 1];
+    a.w_off[l] = (int)g.w_off[l];
+    a.b_off[l] = (int)g.b_off[l];
   }
-  a.n_params = off;
-  a.n_act = act_floats;
+  a.n_params = (int)g.n_params;
+  a.act_off = (int)g.act_off;
+  a.area_smem_off = (int)g.area_smem_off;
+  a.area_bytes = (size_t)g.area_bytes;
   a.batch = opts->batch_size;
   a.epochs = opts->epochs;
   a.optimizer = opts->optimizer;
@@ -365,10 +374,7 @@ extern "C" int fa_mlp_train(int n_layers, const int* dims, const int* activation
   a.given_ranges = in_ranges != nullptr;
   const int d0 = dims[0];
   const size_t J = (size_t)n_jobs, P = (size_t)a.n_params;
-  const int fixed = ((2 * kTrainThreads + 2 * d0 + a.bpad) * (int)sizeof(double) + 3 * a.bpad * (int)sizeof(int) + 15) & ~15;
-  const bool act_smem = fixed + act_floats * (int)sizeof(float) <= kSmemCap;
-  const int smem = act_smem ? fixed + act_floats * (int)sizeof(float) : fixed;
-  a.act_smem_off = fixed;
+  const int smem = (int)g.smem_bytes;
 
   DeviceBuffers buf;
   a.rows = buf.upload(rows, n_rows * d0);
@@ -384,7 +390,7 @@ extern "C" int fa_mlp_train(int n_layers, const int* dims, const int* activation
     if (buf.err == cudaSuccess) buf.err = cudaMemset(a.m1, 0, J * P * sizeof(float));
     if (buf.err == cudaSuccess) buf.err = cudaMemset(a.m2, 0, J * P * sizeof(float));
   }
-  if (!act_smem) a.act_g = buf.alloc<float>(J * (size_t)act_floats);
+  if (!g.area_in_smem) a.area_g = buf.alloc<unsigned char>(J * a.area_bytes);
   a.ranges = in_ranges ? buf.upload(in_ranges, J * 2 * d0) : buf.alloc<double>(J * 2 * d0);
   a.history = buf.alloc<double>(J * (size_t)a.epochs * 2);
   std::vector<int> bad(J, INT_MAX);
