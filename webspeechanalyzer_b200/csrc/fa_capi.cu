@@ -159,6 +159,9 @@ struct fa_handle {
   int k3_workers = 0;    // warps of the epoch-tracking grid
   int k3_impl = 2;       // FA_K3_IMPL: 2 = accumulate_fm2 kernel + redo launch (default), 1 = the general kernel alone
   int k3_warps = 0, k3_regs = 0, k3_finalize_smem = 1;   // FA_K3_WARPS, FA_K3_REGS, FA_K3_FINALIZE_HBM
+  // K3 writes an epoch table + work list, and its rows sit at the epochs' first frames: mode 1, and the utterance-mode scan
+  // whose finalisations run in their own launch (fa_segfin_kernel; not level 3, which finalises in the scan)
+  bool k3_epochs() const { return k3_mode == 1 || (k3_impl == 2 && cfg.output_level != FA_LEVEL_SEGMENTS); }
   bool debug_sync = false;  // FA_DEBUG_SYNC
   int k1a_variant = 0;      // FA_K1A_VARIANT (see fa_launch_spectrum)
   int k1_fused = 0;         // FA_K1_FUSED=1: the fused K1 kernel (fft_size 2048, utterance mode) instead of K1a + K1b.  Measured
@@ -748,6 +751,8 @@ static int prepare(fa_handle* h) {
     if (h->k3_mode == 1) {
       FA_CUDA(h->d_frctl.reserve(Fz * sizeof(unsigned)));
       FA_CUDA(h->d_frv.reserve(Fz * sizeof(double)));
+    }
+    if (h->k3_epochs()) {
       FA_CUDA(h->d_epochs.reserve((Fz + nz) * sizeof(FaEpoch)));
       FA_CUDA(h->d_work.reserve((Fz + nz) * sizeof(int2)));
       FA_CUDA(h->d_k3q.reserve(2 * kMaxSub * sizeof(int)));
@@ -1003,10 +1008,13 @@ static int launch_sub(fa_handle* h, const SubBatch& sb, int slot, cudaStream_t s
     g.no_truncate = h->no_truncate;
     g.impl = h->k3_impl; g.warps_per_cta = h->k3_warps; g.reg_cap = h->k3_regs; g.redo_count = h->d_fix.as<int>() + 2;
     g.mode = h->k3_mode;
-    if (g.mode == 1) {
-      g.fr_ctl = h->d_frctl.as<unsigned>(); g.fr_v = h->d_frv.as<double>(); g.epochs = h->d_epochs.as<FaEpoch>();
+    if (h->k3_epochs()) {
+      g.epochs = h->d_epochs.as<FaEpoch>();
       g.work = h->d_work.as<int2>() + (sb.r0 + sb.u0);      // the sub-batch's slice (capacity: its frames + utterances)
       g.work_count = h->d_k3q.as<int>() + 2 * slot;
+    }
+    if (g.mode == 1) {
+      g.fr_ctl = h->d_frctl.as<unsigned>(); g.fr_v = h->d_frv.as<double>();
       g.n_workers = h->k3_workers;
       if (h->ctl_chunk > 0) {
         const size_t tc = (size_t)h->total_cchunks;
@@ -1033,7 +1041,7 @@ static int launch_sub(fa_handle* h, const SubBatch& sb, int slot, cudaStream_t s
       fp.utt_begin = sb.u0; fp.utt_count = sb.u1 - sb.u0;
       fp.segs = g.segs; fp.n_segs = g.n_segs; fp.syls = g.syls; fp.n_syls = g.n_syls; fp.formants = g.formants;
       fp.features = h->d_features.as<double>(); fp.n_feat = cnt + 4 * n;
-      fp.epochs = h->k3_mode == 1 ? h->d_epochs.as<FaEpoch>() : nullptr;
+      fp.epochs = h->k3_epochs() ? h->d_epochs.as<FaEpoch>() : nullptr;
       // rows of one utterance are spread over `row_slices` CTAs (a one-hour stream has ~2000 rows in ONE utterance)
       fp.row_slices = (int)std::min<long long>(64, std::max<long long>(1, (sb.r1 - sb.r0) / std::max(1, sb.u1 - sb.u0) / 256));
       FA_CUDA(fa_launch_features(fp, s3, &h->launches));
@@ -1042,7 +1050,7 @@ static int launch_sub(fa_handle* h, const SubBatch& sb, int slot, cudaStream_t s
       FaCurveParams cp;
       cp.frame_off = meta + 2 * n; cp.n_utt = n; cp.utt_begin = sb.u0; cp.utt_count = sb.u1 - sb.u0;
       cp.segs = g.segs; cp.n_segs = g.n_segs; cp.syls = g.syls; cp.n_syls = g.n_syls; cp.formants = g.formants; cp.energy = g.energy;
-      cp.epochs = h->k3_mode == 1 ? h->d_epochs.as<FaEpoch>() : nullptr;
+      cp.epochs = h->k3_epochs() ? h->d_epochs.as<FaEpoch>() : nullptr;
       cp.list = h->d_curve_list.as<int2>() + (sb.r0 + sb.u0); cp.list_count = h->d_curve_count.as<int>() + slot;
       cp.list_cap = (sb.r1 - sb.r0) / 2 + (sb.u1 - sb.u0);
       cp.work = h->d_curve_work.as<double>(); cp.status = h->d_curve_status.as<int>();
@@ -1053,7 +1061,7 @@ static int launch_sub(fa_handle* h, const SubBatch& sb, int slot, cudaStream_t s
       FaUtteranceParams up;
       up.frame_off = meta + 2 * n; up.n_utt = n; up.utt_begin = sb.u0; up.utt_count = sb.u1 - sb.u0;
       up.segs = g.segs; up.n_segs = g.n_segs; up.syls = g.syls; up.formants = g.formants;
-      up.epochs = h->k3_mode == 1 ? h->d_epochs.as<FaEpoch>() : nullptr;
+      up.epochs = h->k3_epochs() ? h->d_epochs.as<FaEpoch>() : nullptr;
       up.row_base = meta + 4 * n + 2; up.rows = h->d_features.as<double>(); up.n_feat = cnt + 4 * n; up.overflow = g.overflow;
       FA_CUDA(fa_launch_utterance(up, s3, &h->launches));
     }
@@ -1076,7 +1084,7 @@ static int run_device(fa_handle* h, bool with_h2d, bool with_sink) {
   const long long* meta = h->d_meta.as<long long>();
   h->launches = 0;
   if (c.output_level >= 3) FA_CUDA(cudaMemsetAsync(h->d_counts.p, 0, sizeof(int) * 6 * (size_t)n, s));
-  if (c.output_level >= 3 && h->k3_mode == 1) FA_CUDA(cudaMemsetAsync(h->d_k3q.p, 0, 2 * kMaxSub * sizeof(int), s));
+  if (c.output_level >= 3 && h->k3_epochs()) FA_CUDA(cudaMemsetAsync(h->d_k3q.p, 0, 2 * kMaxSub * sizeof(int), s));
   if (c.output_level == FA_LEVEL_SYL_CURVES) FA_CUDA(cudaMemsetAsync(h->d_curve_count.p, 0, kMaxSub * sizeof(int), s));
   FA_CUDA(cudaMemsetAsync(h->d_fix.p, 0, 3 * sizeof(int), s));
   h->fixups[0] = h->fixups[1] = h->fixups[2] = -1;
@@ -1132,7 +1140,7 @@ static int run_device(fa_handle* h, bool with_h2d, bool with_sink) {
     FaGatherArgs ga;
     ga.feat_width = h->feat_width();
     ga.l3_mult = c.output_level == FA_LEVEL_SEGMENTS ? h->maxp : 0;
-    ga.epochs = h->k3_mode == 1 ? h->d_epochs.as<FaEpoch>() : nullptr;
+    ga.epochs = h->k3_epochs() ? h->d_epochs.as<FaEpoch>() : nullptr;
     ga.row_slices = (int)std::min<long long>(64, std::max<long long>(1, h->total_frames / std::max(1, n) / 256));
     ga.feat_base = c.output_level == FA_LEVEL_UTTERANCE ? meta + 4 * n + 2 : nullptr;
     ga.frame_off = meta + 2 * n; ga.n_utt = n; ga.n_segs = cnt; ga.n_rows = cnt + 2 * n; ga.n_syls = cnt + 3 * n;

@@ -84,14 +84,17 @@ struct FaPeaksParams {
   double* gsum;                  // [F_total] sum e[1..B-1]
 };
 
-// One finalisation of the control scan (K3a -> K3b): the frames of the track epoch that ends in it and the scalar state
-// O() @B27088 reads.  Index in the per-utterance table = index in seg_ci.
+// One finalisation of the control scan (K3a -> K3b), or of the utterance-mode scan (fa_segment2_kernel -> the finaliser): the
+// frames of the track epoch that ends in it and the scalar state O() @B27088 reads.  Index in the per-utterance table = index
+// in seg_ci.  The epoch's points sit in the point pool from (frame_off[u] + first) * maxp on.
 struct __align__(16) FaEpoch {
   int first;                     // first frame of the epoch (frame index inside the utterance): tracks were cleared before it
   int last;                      // last frame to replay (the frame that triggered the finalisation; F - 1 for segment_truncate)
   int n_arg, no_fm_segs, current_frame, c_ci;
   int trk_off, trk_cap;          // the epoch's slice of the utterance's track table (capacity = accepted peaks of the epoch)
   double y, v;                   // thresholds at finalisation
+  double c_energy, s_energy;     // utterance-mode scan only: the tracker's energies at finalisation
+  int n_tr, n_pts;               // ... and its track / point counts (the control scan leaves them to K3b's replay)
 };
 
 // the control state that crosses a chunk boundary of the control scan (K3a stream mode)
@@ -138,7 +141,8 @@ struct FaSegmentParams {
   int mode;
   unsigned* fr_ctl;                   // [F_total] bit 31: the frame reaches accumulate_fm; low bits: its (stale) label c_ci
   double* fr_v;                       // [F_total] gate threshold v after the frame (= v at the start of the next frame)
-  FaEpoch* epochs;                    // [F_total + n_utt] per-utterance tables at base frame_off[u] + u
+  FaEpoch* epochs;                    // [F_total + n_utt] per-utterance tables at base frame_off[u] + u (mode 1, and the
+                                      // finalisations fa_segment2_kernel records at every level but 3)
   int2* work;                         // epoch work list of this sub-batch: (utterance, seg_ci index)
   int* work_count;                    // [2]: entries in the list, next entry to take
   int n_workers;                      // warps of the K3b grid (cs_spill has one slice per worker in mode 1)

@@ -1009,6 +1009,10 @@ __global__ void __launch_bounds__(kBound, 1) fa_segment_kernel(const FaSegmentPa
     p.n_rows[u] = st.n_rows;
     p.n_syls[u] = st.n_syls;
     p.overflow[u] = st.overflow;
+    // redo behind fa_segment2_kernel + fa_segfin_kernel: the consumers find every utterance's rows through the epoch table,
+    // so point it at the dense rows written here
+    if (p.epochs)
+      for (int si = 0; si < st.n_segs; si++) p.epochs[bs.sb + si].first = p.segs[bs.sb + si].row_offset;
   }
 }
 
@@ -1221,6 +1225,27 @@ struct PeakRegs {
   unsigned long long pl, ph;
 };
 
+// O()'s acceptance test at a finalisation of fa_segment2_kernel; an accepted attempt becomes one FaEpoch record (everything
+// finalize_fast / finalize_segment read of the scan state) and one unit of work for fa_segfin_kernel.  The scan itself never
+// reads what a finalisation computes: the next frame only needs seg_reset, and the stored / row / syllable counters only place
+// outputs, which fa_segfix_kernel numbers afterwards.
+__device__ __forceinline__ int finalize_record(const FaSegmentParams& p, ScanState& st, const Bases& bs, const int n_arg,
+                                               const int first, const int last, const int lane) {
+  const int len = n_arg - st.no_fm_segs;
+  if (!(len > p.seg_min_frames && st.c_started >= 2)) return 0;
+  if (lane == 0) {
+    FaEpoch e;
+    e.first = first; e.last = last; e.n_arg = n_arg; e.no_fm_segs = st.no_fm_segs; e.current_frame = st.current_frame;
+    e.c_ci = st.c_ci; e.trk_off = first * p.maxp; e.trk_cap = bs.tcap; e.y = st.y; e.v = st.v;
+    e.c_energy = st.c_energy; e.s_energy = st.s_energy; e.n_tr = st.n_tr; e.n_pts = st.n_pts;
+    p.epochs[bs.sb + st.n_segs] = e;
+    const int w = atomicAdd(p.work_count, 1);
+    p.work[w] = make_int2(bs.u, st.n_segs);
+  }
+  st.n_segs++;
+  return 1;
+}
+
 template <int kBound>
 __global__ void __launch_bounds__(kBound, 1) fa_segment2_kernel(const FaSegmentParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -1232,8 +1257,10 @@ __global__ void __launch_bounds__(kBound, 1) fa_segment2_kernel(const FaSegmentP
   Bases bs;
   bs.row0 = p.frame_off[u];
   bs.F = (int)(p.frame_off[u + 1] - bs.row0);
-  bs.tb = p.track_base[u];
-  bs.tcap = (int)(p.track_base[u + 1] - bs.tb);
+  const long long tb0 = p.track_base[u];
+  const int tcap0 = (int)(p.track_base[u + 1] - tb0);
+  bs.tb = tb0;
+  bs.tcap = tcap0;
   int maxp = p.maxp;
   bs.pb = bs.row0 * maxp;
   bs.sb = bs.row0 + u;
@@ -1241,6 +1268,18 @@ __global__ void __launch_bounds__(kBound, 1) fa_segment2_kernel(const FaSegmentP
   bs.u = u;
   bs.spill = u;
   const unsigned lt = (1u << lane) - 1u;
+  // Finalisations are recorded (finalize_record) and run by fa_segfin_kernel behind the scan; every epoch then owns the slices
+  // of the track table and the point pool that start at its first frame (an epoch of f frames needs at most f * maxp entries
+  // of each).  Level 3 (the raw-track export, tables at the utterance's point-pool base) still finalises in the chain.
+  const bool defer = p.level != 3;
+  int epoch_first = 0;
+  auto new_epoch = [&](const int t) {
+    if (!defer) return;
+    epoch_first = t;
+    bs.tb = tb0 + (long long)t * maxp;
+    bs.tcap = tcap0 - t * maxp;
+    bs.pb = (bs.row0 + t) * maxp;
+  };
 
   ScanState st;
   st.current_frame = 0; st.no_fm_segs = 0; st.c_ci = 0; st.c_started = -1; st.w = 0; st.k = 0;
@@ -1344,30 +1383,33 @@ __global__ void __launch_bounds__(kBound, 1) fa_segment2_kernel(const FaSegmentP
       bool strong;                                                  // h (n - 1) / (d - h) > 4
       if (p.auto_gate) strong = d > h && h * (double)(n - 1) > 4 * (d - h);
       else strong = (d > h ? h * (double)(n - 1) / (d - h) : 0) > 4;
-      if (n > 0 && pbin > 7 && pbin < p.max_voiced_bin && n > 4 && strong) { seg_reset(st, S, 0, lane); st.c_started = 0; }
-      else st.no_fm_segs++;
+      if (n > 0 && pbin > 7 && pbin < p.max_voiced_bin && n > 4 && strong) {
+        seg_reset(st, S, 0, lane); st.c_started = 0; new_epoch(t);
+      } else st.no_fm_segs++;
     }
     if (st.c_started >= 0) {
       if (n == 0 || pbin < 7 || pbin >= p.max_voiced_bin || (n > 3 && weak)) {
         st.no_fm_segs++;
         if (st.c_started < 2) st.c_started--;
-        else if ((double)st.no_fm_segs >= p.seg_breaker) fin = finalize_copy(p, S, st, bs, st.c_ci + 1, lane);
-        else if (p.auto_gate) noise_gate(st, S, h, lane);
+        else if ((double)st.no_fm_segs >= p.seg_breaker)
+          fin = defer ? finalize_record(p, st, bs, st.c_ci + 1, epoch_first, t, lane) : finalize_copy(p, S, st, bs, st.c_ci + 1, lane);
+        else if (p.auto_gate && gate_update(st, h)) { seg_reset(st, S, 0, lane); new_epoch(t); }
       } else {
-        if (p.auto_gate) noise_gate(st, S, h, lane);
+        if (p.auto_gate && gate_update(st, h)) { seg_reset(st, S, 0, lane); new_epoch(t); }
         accumulate_fm2(p, S, st, bs, pr.m, pr.pkd, pr.amp, pr.pl, pr.ph, t_stale, g, st.v, lane);
         if (st.c_started < 2) st.c_started++; else st.no_fm_segs = 0;
       }
     }
     st.c_ci++;
     if (fin != -2) {
-      S.t_wm[lane] = 0u; S.t_wm[lane + 32] = 0u;   // the finalisation used the track slots as scratch
       seg_reset(st, S, -1, lane);                  // the promise's micro-task runs before the next frame
+      new_epoch(t + 1);
     }
   }
   // segment_truncate @B30800 (not for the prefix of a stream that is still running: fa_set_truncate)
   if (!st.overflow && !p.no_truncate) {
-    finalize_copy(p, S, st, bs, st.c_ci, lane);
+    if (defer) finalize_record(p, st, bs, st.c_ci, epoch_first, bs.F - 1, lane);
+    else finalize_copy(p, S, st, bs, st.c_ci, lane);
     seg_reset(st, S, 1, lane);
   }
   if (lane == 0) {
@@ -2151,6 +2193,267 @@ __global__ void __launch_bounds__(kBound, 1) fa_segtrack_kernel(const FaSegmentP
   }
 }
 
+// =====================================================================================================================
+// The finaliser of the utterance-mode scan: O() @B27088 for every FaEpoch record fa_segment2_kernel wrote, one CTA per
+// record (a persistent grid pulls them from the work list).  Every thread takes part in staging and ranking the eligible
+// tracks, counting the selected points per row and scattering their sort keys and payloads (bin / span, energy) into shared
+// memory, row by row; after that the record needs no global load: the apply runs one thread per row, the syllable scan one
+// warp.  Only the SELECTED points are staged (most tracks are one-point noise tracks that get no slot), 20 B each.  The
+// arithmetic and its order are finalize_fast's: count-smaller ranking with the creation-order tie rule, the sequential slot
+// rule of straighten_formants, visits in (rank, ordinal) order -- a key (rank, ordinal) is unique, so the per-row selection
+// sort needs no pool order --, the float / double accumulation of g0..g2 row by row, sep_syllables, and the thrown segment
+// (stored = -1, still counted).  Rows and syllables land in the epoch's own frame range, as K3b's do; fa_segfix_kernel
+// numbers them.  A record whose tables do not fit kFinSmem (or every record with finalize_in_smem = 0) is finalised by warp
+// 0 with finalize_segment in HBM.
+// =====================================================================================================================
+constexpr int kFinThreads = 256;
+constexpr int kFinSmem = 64 * 1024;   // 3 CTAs per SM
+
+__global__ void __launch_bounds__(kFinThreads, 3) fa_segfin_kernel(const FaSegmentParams p) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  __shared__ int s_wi, s_nr, s_nsel, s_thrown, s_wsum[kFinThreads / 32];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const unsigned lt = (1u << lane) - 1u;
+  const int maxp = p.maxp;
+  const int n_work = *reinterpret_cast<volatile int*>(p.work_count);
+  for (;;) {
+    if (tid == 0) s_wi = atomicAdd(p.work_count + 1, 1);
+    __syncthreads();
+    const int wi = s_wi;
+    __syncthreads();   // every thread has read s_wi before thread 0 takes the next item
+    if (wi >= n_work) break;
+    const int2 wk = p.work[wi];
+    const int u = wk.x;
+    if (p.overflow[u]) continue;        // handed to the general kernel (2) or failed (1): nothing of it is kept
+    const FaEpoch E = p.epochs[p.frame_off[u] + u + wk.y];
+    Bases bs;
+    bs.row0 = p.frame_off[u];
+    bs.F = (int)(p.frame_off[u + 1] - bs.row0);
+    bs.sb = bs.row0 + u;
+    bs.tb = p.track_base[u] + E.trk_off;
+    bs.tcap = E.trk_cap;
+    bs.pb = (bs.row0 + E.first) * maxp;
+    bs.rb = bs.sb + E.first;
+    bs.u = u;
+    bs.spill = 0;
+    const int T = E.n_tr, NP = E.n_pts, len = E.n_arg - E.no_fm_segs;
+    auto in_hbm = [&]() {
+      if (warp == 0) {
+        ScanState st;
+        st.current_frame = E.current_frame; st.no_fm_segs = E.no_fm_segs; st.c_ci = E.c_ci; st.c_started = 2; st.w = 0; st.k = 0;
+        st.y = E.y; st.v = E.v; st.x = E.y; st.v0 = E.v; st.T = 0; st.s_energy = E.s_energy; st.c_energy = E.c_energy;
+        st.n_tr = T; st.n_pts = NP; st.n_slots = 0;
+        st.n_segs = wk.y; st.n_stored = 0; st.n_rows = E.first; st.n_syls = E.first; st.overflow = 0;
+        finalize_segment(p, st, bs, E.n_arg, lane);
+      }
+    };
+    // layout: rc, ro, fill i32[len] | rank i16[T] | slot i8[T] | cmean f64[nr] | cidx i32[nr] | order i16[nr] |
+    //         key u64[n_sel] | e f64[n_sel] | binspan i32[n_sel]     (nr: eligible tracks, n_sel: selected points)
+    const int off_tr = 12 * len, off_c = (off_tr + 3 * T + 7) & ~7;
+    if (!p.finalize_in_smem || off_c > kFinSmem) { in_hbm(); continue; }
+    int* rc = reinterpret_cast<int*>(smem_raw);
+    int* ro = rc + len;
+    int* fill = ro + len;
+    short* rank = reinterpret_cast<short*>(smem_raw + off_tr);
+    signed char* slot = reinterpret_cast<signed char*>(rank + T);
+    const double vmin = E.v;
+    // ---- get_ranked_formants @B35670: count >= 2, mean >= 7, stable ascending by mean ----
+    for (int i = tid; i < T; i += kFinThreads) {
+      const double m = p.trk_sum_eb[bs.tb + i] / p.trk_sum_e[bs.tb + i];
+      slot[i] = p.trk_count[bs.tb + i] >= 2 && m >= 7 ? 1 : -1;    // eligible (slot assigned below)
+    }
+    for (int r = tid; r < len; r += kFinThreads) { rc[r] = 0; fill[r] = 0; }
+    if (tid == 0) { s_nr = 0; s_nsel = 0; s_thrown = 0; }
+    __syncthreads();
+    {
+      int cnt = 0;
+      for (int i = tid; i < T; i += kFinThreads) cnt += slot[i] > 0;
+      cnt = __reduce_add_sync(FULL, cnt);
+      if (lane == 0 && cnt) atomicAdd(&s_nr, cnt);
+    }
+    __syncthreads();
+    const int nr = s_nr;
+    const int off_i = off_c + 8 * nr, off_o = off_i + 4 * nr, off_k = (off_o + 2 * nr + 7) & ~7;
+    if (off_k > kFinSmem) { in_hbm(); continue; }
+    double* cmean = reinterpret_cast<double*>(smem_raw + off_c);
+    int* cidx = reinterpret_cast<int*>(smem_raw + off_i);
+    short* order = reinterpret_cast<short*>(smem_raw + off_o);
+    // the eligible tracks compacted in creation order (block-wide scan of the flags, 256 tracks at a time)
+    for (int i0 = 0, base = 0; i0 < T; i0 += kFinThreads) {
+      const int i = i0 + tid;
+      const bool elig = i < T && slot[i] > 0;
+      const unsigned em = __ballot_sync(FULL, elig);
+      if (lane == 0) s_wsum[warp] = __popc(em);
+      __syncthreads();
+      int pre = base, tot = 0;
+      for (int w = 0; w < kFinThreads / 32; w++) { if (w < warp) pre += s_wsum[w]; tot += s_wsum[w]; }
+      if (elig) {
+        const int k = pre + __popc(em & lt);
+        cmean[k] = p.trk_sum_eb[bs.tb + i] / p.trk_sum_e[bs.tb + i];
+        cidx[k] = i;
+        slot[i] = -1;
+      }
+      base += tot;
+      __syncthreads();
+    }
+    for (int k = tid; k < nr; k += kFinThreads) {
+      const double m = cmean[k];
+      int rk = 0;
+      for (int j = 0; j < nr; j++) {
+        const double mj = cmean[j];
+        rk += (mj < m || (mj == m && j < k)) ? 1 : 0;   // the compacted list keeps the tracks in creation order
+      }
+      rank[cidx[k]] = (short)rk;
+      order[rk] = (short)k;
+    }
+    __syncthreads();
+    // ---- slot assignment of straighten_formants @B35074 (sequential over the ranking) ----
+    if (tid == 0) {
+      double anchor = 0;
+      int sl = 0;
+      for (int r = 0; r < nr; r++) {
+        const int k = order[r];
+        const double m = cmean[k];
+        if (fabs(m - anchor) > 20) {
+          anchor = m;
+          sl++;
+          if (sl >= 3) break;
+        }
+        slot[cidx[k]] = (signed char)sl;
+      }
+    }
+    __syncthreads();
+    // ---- rows: count the selected points of every row; a selected point outside the segment throws ----
+    {
+      bool thrown = false;
+      int nsel = 0;
+      for (int q = tid; q < NP; q += kFinThreads) {
+        const int i = __ldg(p.pt_track + bs.pb + q), fr = __ldg(p.pt_frame + bs.pb + q);
+        if (slot[i] >= 0) {
+          if (fr < 0 || fr >= len) thrown = true;   // r[d] is undefined -> TypeError -> .catch(L(-1))
+          else { atomicAdd(&rc[fr], 1); nsel++; }
+        }
+      }
+      if (thrown) s_thrown = 1;
+      nsel = __reduce_add_sync(FULL, nsel);
+      if (lane == 0 && nsel) atomicAdd(&s_nsel, nsel);
+    }
+    __syncthreads();
+    fa_segment seg;
+    seg.start = E.current_frame - len; seg.len = len; seg.stored = -1; seg.n_syllables = 0; seg.first_syllable = -1;
+    seg.row_offset = -1; seg.ymax = E.y; seg.vmin = E.v; seg.cs_ratio = E.c_energy / E.s_energy;
+    if (s_thrown) {
+      if (tid == 0) p.segs[bs.sb + wk.y] = seg;
+      continue;
+    }
+    const int n_sel = s_nsel;
+    if (off_k + 20 * n_sel > kFinSmem) { in_hbm(); continue; }
+    unsigned long long* key = reinterpret_cast<unsigned long long*>(smem_raw + off_k);
+    double* pe = reinterpret_cast<double*>(key + n_sel);
+    int* bsp = reinterpret_cast<int*>(pe + n_sel);
+    if (warp == 0) {   // exclusive prefix of the row counts
+      int run = 0;
+      for (int r0 = 0; r0 < len; r0 += 32) {
+        const int r = r0 + lane;
+        const int c = r < len ? rc[r] : 0;
+        int incl = c;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+          const int t = __shfl_up_sync(FULL, incl, o);
+          if (lane >= o) incl += t;
+        }
+        if (r < len) ro[r] = run + incl - c;
+        run += __shfl_sync(FULL, incl, 31);
+      }
+    }
+    __syncthreads();
+    // key = rank << 42 | ordinal << 22 | staged index << 2 | slot  (ordinal < 2^20 points, staged index < 2^20, slot < 3)
+    for (int q = tid; q < NP; q += kFinThreads) {
+      const int i = __ldg(p.pt_track + bs.pb + q);
+      const int sl = slot[i];
+      if (sl >= 0) {
+        const int fr = __ldg(p.pt_frame + bs.pb + q), od = __ldg(p.pt_ord + bs.pb + q);
+        const int pos = ro[fr] + atomicAdd(&fill[fr], 1);
+        key[pos] = ((unsigned long long)rank[i] << 42) | ((unsigned long long)od << 22) | ((unsigned long long)pos << 2) |
+                   (unsigned long long)sl;
+        pe[pos] = __ldg(p.pt_e + bs.pb + q);
+        bsp[pos] = __ldg(p.pt_binspan + bs.pb + q);
+      }
+    }
+    __syncthreads();
+    // ---- apply: thread per row, points in (track rank, point ordinal) order ----
+    float* Fout = p.formants + (size_t)(bs.row0 + E.first) * 9;
+    float* Eout = p.energy + (size_t)(bs.row0 + E.first) * 3;
+    for (int fr = tid; fr < len; fr += kFinThreads) {
+      const int k = rc[fr], off = ro[fr];
+      float f0 = 0, f1 = 0, f2 = 0, f3 = 0, f4 = 0, f5 = 0, f6 = 0, f7 = 0, f8 = 0, g0 = 0, g1 = 0, g2 = 0;
+      long long last = -1;
+      for (int it = 0; it < k; it++) {
+        long long bestkey = 0x7fffffffffffffffll;
+        for (int z = 0; z < k; z++) {
+          const long long kz = (long long)key[off + z];
+          if (kz > last && kz < bestkey) bestkey = kz;
+        }
+        last = bestkey;
+        const int bq = (int)((bestkey >> 2) & 0xfffffu);
+        int sl = (int)(bestkey & 3u);
+        const int bs_ = bsp[bq];
+        const int bin = bs_ & 0xff, span = bs_ >> 16;   // bits 8..15: the point's lower bound (level 3)
+        const double Ep = pe[bq];
+        const float cur = sl == 0 ? f0 : sl == 1 ? f3 : f6;
+        if ((double)cur > vmin && (double)cur < (double)bin && sl < 2) sl++;
+        const float fb = (float)bin, fe = (float)Ep, fs = (float)span;
+        if (sl == 0) { f0 = fb; f1 = fe; f2 = fs; }
+        else if (sl == 1) { f3 = fb; f4 = fe; f5 = fs; }
+        else { f6 = fb; f7 = fe; f8 = fs; }
+        g0 = (float)((double)g0 + (double)bin * Ep);
+        g1 = (float)((double)g1 + Ep);
+        g2 = (float)((double)g2 + (double)span * Ep);
+      }
+      float* fo = Fout + (size_t)fr * 9;
+      fo[0] = f0; fo[1] = f1; fo[2] = f2; fo[3] = f3; fo[4] = f4; fo[5] = f5; fo[6] = f6; fo[7] = f7; fo[8] = f8;
+      float* eo = Eout + (size_t)fr * 3;
+      eo[0] = g0; eo[1] = g1; eo[2] = g2;
+      fill[fr] = (double)g1 > vmin ? 1 : 0;   // sep_syllables needs "energy > vmin" per row
+    }
+    __syncthreads();
+    if (warp != 0) continue;
+    // ---- sep_syllables @B34757 (provisional: stored_seg 0, syllables from the epoch's first frame on) ----
+    int nsyl = 0;
+    if (p.level == 10 || p.level == 11 || p.level == 12 || p.level == 13) {
+      int sstart = -1, quiet = 0, loud = 0;
+      for (int e0 = 0; e0 < len; e0 += 32) {
+        const int e = e0 + lane;
+        const bool is_loud = e < len && fill[e] != 0;
+        const unsigned bits = __ballot_sync(FULL, is_loud);
+        const int cnt = min(32, len - e0);
+        for (int b = 0; b < cnt; b++) {
+          const int ee = e0 + b;
+          if ((bits >> b) & 1u) { quiet = 0; loud++; if (sstart < 0) sstart = ee; }
+          else quiet++;
+          if ((loud > 20 && quiet > 0) || (loud > 10 && quiet > 1) || (loud > 0 && quiet > 4) || (ee >= len - 1 && loud > 4)) {
+            const int end = ee - quiet;
+            if (end - sstart > 1) {
+              if (lane == 0) {
+                fa_syllable sy;
+                sy.stored_seg = 0; sy.start = sstart; sy.len = end - sstart; sy.reserved = 0;
+                p.syls[bs.sb + E.first + nsyl] = sy;
+              }
+              nsyl++;
+              sstart = -1;
+              loud = 0;
+            }
+          }
+        }
+      }
+    }
+    if (lane == 0) {
+      seg.stored = 0; seg.row_offset = E.first; seg.first_syllable = E.first; seg.n_syllables = nsyl;
+      p.segs[bs.sb + wk.y] = seg;
+    }
+  }
+}
+
 __global__ void __launch_bounds__(kCtlWarps * 32) fa_segfix_kernel(const FaSegmentParams p) {
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   const int ui = blockIdx.x * kCtlWarps + wib;
@@ -2264,6 +2567,15 @@ cudaError_t fa_launch_segment(const FaSegmentParams& p_in, cudaStream_t s, int* 
     p.smem_per_warp = full;
     if (launches) (*launches)++;
     if (e != cudaSuccess) return e;
+    if (p.level != 3) {   // the recorded finalisations, then the numbering of the stores (level 3 finalised in the chain)
+      e = cudaFuncSetAttribute(fa_segfin_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFinSmem);
+      if (e != cudaSuccess) return e;
+      fa_segfin_kernel<<<num_sms * 3, kFinThreads, kFinSmem, s>>>(p);
+      fa_segfix_kernel<<<(p.utt_count + kCtlWarps - 1) / kCtlWarps, kCtlWarps * 32, 0, s>>>(p);
+      if (launches) (*launches) += 2;
+      e = cudaGetLastError();
+      if (e != cudaSuccess) return e;
+    }
     p.redo_only = 1;   // whatever fa_segment2_kernel handed back (overflow == 2): normally nothing, every warp exits at once
   } else {
     p.redo_only = 0;
